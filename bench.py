@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- enhanced audio-seconds per second of the N-step bridge sampler hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the whole hot path (fused STFT+compress+pad -> 5-step SB/ode_ei sampler on
 the NCSN++ backbone -> fused decompress+iSTFT) over the batch of 256 synthetic 4 s / 16 kHz utterances
@@ -40,6 +40,24 @@ BRIDGE_STEPS = 5
 GFLOP_PER_FORWARD = 532.1          # SURVEY.md section 8(d): one ncsnpp_v2 forward on a 4 s utterance (2*MAC)
 METRIC = "enhanced audio-sec/sec (5-step SB bridge, ncsnpp_v2)"
 UNIT = "audio-s/s"
+DUMP_BYTES = 60 * 2 ** 20          # --dump-outputs: stays under 64 MB with room for the .npy headers and row lists
+
+
+def dump_output(out_dir, name, t, utt_ids=None):
+    """--dump-outputs: tensor `t` as out_dir/<name>.npy in float32, so that the outputs of two builds can be compared one for one.
+    For per-utterance rows, `utt_ids` names the utterance of each row and goes to out_dir/<name>_rows.npy; more rows than
+    DUMP_BYTES holds are cut to a fixed, seeded sample (the same rows for the same ids, whatever the build)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    a = t.detach().to("cpu", torch.float32).numpy()
+    if utt_ids is not None:
+        ids = np.asarray(utt_ids, dtype=np.float64)
+        if a.nbytes > DUMP_BYTES:                    # one row fits: main() refuses longer utterances
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_BYTES // (a.nbytes // a.shape[0]), replace=False))
+            a, ids = a[rows], ids[rows]
+        np.save(os.path.join(out_dir, f"{name}_rows.npy"), ids)
+    np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def set_workload(seconds, steps, predictive):
@@ -346,22 +364,25 @@ def train_main(args):
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        out = fn()                                   # the last step's result, for --dump-outputs
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     for _ in range(max(args.warmup, 3)):
         step_device()
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
-    ms = timed(step_device, args.steps)
-    ms_e2e = timed(step_e2e, args.steps)
+    ms, loss = timed(step_device, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_output(args.dump_outputs, "loss", loss)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     # a few 56 ms steps end before nvidia-smi prints its first line: the sampler covers both timed regions (same step, same load)
     clock_info = clocks.stop() if rank == 0 else None
     # phase split of one step (events around forward / backward / optimiser)
@@ -418,7 +439,6 @@ def tfgridnet_main(args):
     dev = torch.device("cuda:0")
     torch.cuda.set_device(dev)
     _lib.check(_lib.load().fdbm_check_device(), "fdbm_check_device")
-    torch.manual_seed(0)
     if pred:
         model = PredictiveEnhancementModel("tfgridnet_5l32c100_predictive")
     else:
@@ -446,19 +466,22 @@ def tfgridnet_main(args):
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        out = fn()                                   # the last step's result, for --dump-outputs
         e1.record()
         torch.cuda.synchronize()
-        return e0.elapsed_time(e1)
+        return e0.elapsed_time(e1), out
 
     for _ in range(max(args.warmup, 3)):
         step_device()
     clocks = ClockSampler(0)
     clocks.start()
-    ms = timed(step_device, args.steps)
+    ms, enhanced = timed(step_device, args.steps)
     clock_info = clocks.stop()
-    ms_e2e = timed(step_e2e, args.steps)
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "enhanced", enhanced, range(args.utts))
+    ms_e2e, _ = timed(step_e2e, args.steps)
     n_fwd = 1 if pred else BRIDGE_STEPS
     T, Q = 256, 257
     # algorithmic MACs of the ten BiLSTM sweeps of one forward (input + recurrent projections + ConvTranspose1d), per utterance
@@ -563,9 +586,21 @@ def main():
                     help="multi-GPU: 'strong' = --utts utterances in TOTAL, sharded (BASELINE configs[1]); 'weak' = --utts per GPU")
     ap.add_argument("--no-gather", action="store_true", help="skip the final NCCL all_gather of the enhanced waveforms")
     ap.add_argument("--no-torch-gpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (enhanced waveforms; the loss for --workload "
+                         "train) to DIR/<name>.npy in float32, a seeded sample of the rows where it exceeds 60 MiB; "
+                         "DIR/<name>_rows.npy names the utterance of each row")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 20 if args.workload == "train" else 3
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "files"):
+        ap.error("--dump-outputs covers the CUDA path of the in-memory workloads (not --impl reference or --workload files)")
+    if args.dump_outputs and args.workload != "train" and int(SR * args.seconds) * 4 > DUMP_BYTES:
+        ap.error(f"--dump-outputs: one {args.seconds:g} s utterance is more than the {DUMP_BYTES} bytes a dump may take")
+    import torch
+    torch.manual_seed(0)             # the Fourier-feature weights are drawn at construction: same arguments, same model and inputs
     predictive = args.workload == "predictive"
     set_workload(args.seconds, args.bridge_steps, predictive)
     if args.workload == "train":
@@ -657,24 +692,28 @@ def main():
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        out = fn()                                   # the last step's result, for --dump-outputs
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     for _ in range(max(args.warmup, 3)):
         step_device()
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
-    ms_total = timed(step_device, args.steps)
+    ms_total, enhanced = timed(step_device, args.steps)
     clock_info = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_output(args.dump_outputs, "enhanced", enhanced, range(total_utts) if do_gather else my_ids)
+    del enhanced
     step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
 
     audio_s = total_utts * UTT_SECONDS
     value = audio_s * args.steps / (ms_total * 1e-3)

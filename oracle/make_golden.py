@@ -10,6 +10,7 @@ The GPU box never runs this; it only reads the committed fixtures.
 """
 from __future__ import annotations
 
+import argparse
 import os
 import sys
 import types
@@ -489,8 +490,97 @@ def variant_goldens(BackboneRegistry=None):
     np.savez_compressed(os.path.join(OUT, "ncsnpp_nf96_T64.npz"), **out)
 
 
+DROPIN_PATHS = {"sb_bb": ("sb", dict(noise_schedule="bb")), "sb_ve": ("sb", dict(noise_schedule="ve")),
+                "sb_vp": ("sb", dict(noise_schedule="vp", c=0.3)), "sb_gmax": ("sb", dict(noise_schedule="gmax")), "fm_ot": ("fm", dict())}
+DROPIN_T = [0.03, 0.2, 0.55, 0.9999, 1.0]
+DROPIN_PC = [(c, k, p) for c, k in (("ald", 1), ("langevin", 2), ("none", 1)) for p in ("euler_maruyama", "none")]
+
+
+def argparse_defaults(cls):
+    pa = argparse.ArgumentParser()
+    cls.add_argparse_args(pa)
+    return vars(pa.parse_args([]))
+
+
+def dropin_soup(backbone_defaults):
+    """The kwargs dictionary train.py hands a backbone (model.py:47-48 passes the values of ALL argparse groups at once)."""
+    return dict(backbone_defaults, lr=1e-4, ema_decay=0.999, N=5, T=1.0, sampler_type="ode_ei", noise_schedule="bb",
+                base_dir="/x", batch_size=8, n_fft=512, hop_length=256, gpus=1, loss_type="data_prediction_hybrid")
+
+
+def dropin_bridge_inputs():
+    g = torch.Generator().manual_seed(1)
+    return tuple(torch.view_as_complex(torch.randn(5, 1, 9, 4, 2, generator=g)) for _ in range(3))     # s, y, x
+
+
+def dropin_sampler_inputs():
+    """A cheap stand-in model (B = 1, as the reference's broadcasting requires), its conditioning and a fixed noise sequence."""
+    g = torch.Generator().manual_seed(3)
+    y = torch.view_as_complex(torch.randn(1, 1, 17, 8, 2, generator=g)) * 0.3
+    zs = [torch.view_as_complex(torch.randn(1, 1, 17, 8, 2, generator=g)) * 0.5 ** 0.5 for _ in range(40)]
+    model = lambda x, yy, t: 0.6 * x + 0.3 * yy * torch.cos(t)[:, None, None, None] + 0.05 * x.abs()
+    return y, zs, model
+
+
+def dropin_record(Bridge, BackboneRegistry, SpecsDataModule):
+    """What tests/test_reference_dropin.py compares against the original project's objects, computed with the classes given:
+    argparse defaults, state_dict layout, requires_grad flags and per-tensor init statistics of the backbones, Bridge attributes
+    and the scalar path maths on seeded inputs, pc / ode_int sampler outputs with a stand-in model, SpecsDataModule attributes.
+    Returns {name: array}; the JSON-able facts are one JSON string under "meta"."""
+    import itertools
+    import json
+    meta, out = {}, {}
+    cls = BackboneRegistry.get_by_name("ncsnpp_v2")
+    meta["ncsnpp_v2_args"] = argparse_defaults(cls)
+    net = cls(**dropin_soup(meta["ncsnpp_v2_args"]))
+    meta["ncsnpp_v2_shapes"] = {k: list(v.shape) for k, v in net.state_dict().items()}
+    meta["ncsnpp_v2_requires_grad"] = [[n, p.requires_grad] for n, p in net.named_parameters()]
+    torch.manual_seed(0)
+    meta["ncsnpp_v2_init_std"] = {n: float(p.detach().std()) for n, p in cls().named_parameters() if p.numel() > 4096}
+    meta["ncsnpp_v2_predictive_shapes"] = {k: list(v.shape) for k, v in
+                                           BackboneRegistry.get_by_name("ncsnpp_v2_predictive")().state_dict().items()}
+    meta["bridge_args"] = argparse_defaults(Bridge)
+    s, y, x = dropin_bridge_inputs()
+    t, t1 = torch.tensor(DROPIN_T), torch.tensor([0.4])
+    for tag, (path, kw) in DROPIN_PATHS.items():
+        b = Bridge(path, N=7, sampler_type="sde_ei", sampling_eps=1e-3, **kw)
+        meta[tag] = {"attrs": {a: getattr(b, a) for a in ("N", "T", "sampler_type", "start_time", "end_time")},
+                     "sampling_direction": b.path.sampling_direction, "path_T": b.path.T, "path_args": argparse_defaults(type(b.path))}
+        vals = {"path_param": b.path.path_param(t), "std": [b._std(t)], "probability_path": b.probability_path(s, y, t),
+                "score_fn": [b.score_fn(t, x, s, y)], "ode": [b.path.ode(t1, x[:1], s[:1], y[:1])]}
+        if path == "sb":
+            vals.update(sde=b.path.sde(t1, x[:1], s[:1], y[:1]), auxiliary_param=b.path.auxiliary_param(t1),
+                        sampling_param_ode_ei=b.path.sampling_param_ode_ei(t1 * 0.5, t1, 1, "cpu"),
+                        sampling_param_sde_ei=b.path.sampling_param_sde_ei(t1 * 0.5, t1, 1, "cpu"))
+        for name, vs in vals.items():
+            for i, v in enumerate(vs):
+                out[f"{tag}_{name}_{i}"] = c2n(torch.as_tensor(v))
+    y, zs, model = dropin_sampler_inputs()
+    for corrector, steps, predictor in DROPIN_PC:
+        with fixed_noise(zs):
+            out[f"pc_{corrector}_{predictor}"] = c2n(Bridge("sb", N=4, sampler_type="pc").sampler(
+                model, y, predictor_name=predictor, corrector_name=corrector, snr=0.3, corrector_steps=steps))
+    with fixed_noise(itertools.repeat(zs[0])):
+        out["ode_int_fm"] = c2n(Bridge("fm", sampler_type="ode_int").sampler(model, y, rtol=1e-6, atol=1e-6))
+    dm = SpecsDataModule(base_dir="/unused", n_fft=512, hop_length=256, num_frames=256, window="sqrthann", gpu=False)
+    meta["data_module"] = {a: getattr(dm, a) for a in ("normalize", "n_fft", "hop_length", "num_frames", "spec_factor",
+                                                        "spec_abs_exponent", "transform_type")}
+    meta["data_module_stft_kwargs"] = sorted(dm.stft_kwargs)
+    out["data_module_window"] = c2n(dm.window)
+    out["meta"] = np.array(json.dumps(meta, sort_keys=True))
+    return out
+
+
+def dropin_goldens():
+    """(8) tests/golden/dropin.npz: dropin_record run on the original project's Bridge, BackboneRegistry and SpecsDataModule."""
+    Bridge, BackboneRegistry, SpecsDataModule = import_reference()[:3]
+    np.savez_compressed(os.path.join(OUT, "dropin.npz"), **dropin_record(Bridge, BackboneRegistry, SpecsDataModule))
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "tfgridnet":
+    if len(sys.argv) > 1 and sys.argv[1] == "dropin":
+        dropin_goldens()
+    elif len(sys.argv) > 1 and sys.argv[1] == "tfgridnet":
         os.makedirs(OUT, exist_ok=True)
         tfgridnet_goldens()
     elif len(sys.argv) > 1 and sys.argv[1] == "mel":

@@ -1,71 +1,71 @@
-"""The Python seams of the drop-in boundary, checked against the REFERENCE's own objects (CPU, no CUDA call).
+"""The Python seams of the drop-in boundary, checked against what the REFERENCE's own objects give (CPU, no CUDA call).
 
-Runs only where /root/reference is present (the build container); the GPU box has no copy of the reference.
+tests/golden/dropin.npz holds those values (oracle/make_golden.py `dropin`, seeded inputs): argparse defaults, state_dict layout,
+requires_grad flags and init statistics of the backbones, Bridge attributes and path maths, pc / ode_int sampler outputs of a
+stand-in model, SpecsDataModule attributes.  With FDBM_REFERENCE naming a checkout of the original project,
+test_golden_matches_the_reference also recomputes them from its classes and checks registry / state_dict interchange live.
 SURVEY.md section 8(b): (1) BackboneRegistry.register / get_by_name + add_argparse_args + **kwargs tolerance,
 (2) Bridge attributes and path maths, (3) SpecsDataModule attributes, state_dict compatibility in both directions."""
-import argparse
+import json
 import os
-import sys
 
+import numpy as np
 import pytest
 import torch
 
-REF = os.environ.get("FDBM_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "fdbm")), reason="reference checkout not present")
+import make_golden as MG
+from helpers import load_npz
+
+REF = os.environ.get("FDBM_REFERENCE")
 
 
 @pytest.fixture(scope="module")
-def ref():
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
-    import make_golden as MG
-    Bridge, BackboneRegistry, SpecsDataModule, pad_spec, si_sdr = MG.import_reference()
-    import fdbm.bridge as ref_bridge
-    return dict(Bridge=Bridge, BackboneRegistry=BackboneRegistry, SpecsDataModule=SpecsDataModule, pad_spec=pad_spec,
-                si_sdr=si_sdr, bridge_mod=ref_bridge)
+def golden(golden_dir):
+    g = load_npz(os.path.join(golden_dir, "dropin.npz"))
+    return json.loads(str(g.pop("meta"))), g
 
 
-def test_our_backbones_register_into_the_reference_registry(ref):
+def as_json(x):
+    return json.loads(json.dumps(x))
+
+
+def test_our_backbones_register_into_the_reference_registry(golden):
     """`BackboneRegistry.register(name)(cls)` + `get_by_name(name)(**kwargs)` (util/registry.py:17-30, model.py:47-48) with the
-    kwargs soup train.py passes (every argparse group's values at once)."""
+    kwargs soup train.py passes (every argparse group's values at once), and the reference's flags, state_dict layout,
+    parameter flags and initialisation law."""
     import fdbm_b200
-    R = ref["BackboneRegistry"]
-    ref_cls = R.get_by_name("ncsnpp_v2")
+    meta, _ = golden
+    R = fdbm_b200.BackboneRegistry
     R.register("ncsnpp_v2_b200")(fdbm_b200.NCSNpp_v2)
     R.register("ncsnpp_v2_predictive_b200")(fdbm_b200.NCSNpp_v2_predictive)
     cls = R.get_by_name("ncsnpp_v2_b200")
     assert cls is fdbm_b200.NCSNpp_v2
     # argparse seam (train.py:92-93): same flags, same defaults
-    pa, pb = argparse.ArgumentParser(), argparse.ArgumentParser()
-    ref_cls.add_argparse_args(pa); cls.add_argparse_args(pb)
-    assert vars(pa.parse_args([])) == vars(pb.parse_args([]))
+    assert as_json(MG.argparse_defaults(cls)) == meta["ncsnpp_v2_args"]
     # constructor tolerates the reference's full kwargs dictionary (model.py:47-48 passes **kwargs of ALL groups)
-    soup = dict(vars(pa.parse_args([])), lr=1e-4, ema_decay=0.999, N=5, T=1.0, sampler_type="ode_ei", noise_schedule="bb",
-                base_dir="/x", batch_size=8, n_fft=512, hop_length=256, gpus=1, loss_type="data_prediction_hybrid")
-    ours = cls(**soup)
-    theirs = ref_cls(**soup)
+    ours = cls(**MG.dropin_soup(meta["ncsnpp_v2_args"]))
     # state_dict compatibility in both directions, strict
-    sd_ref = theirs.state_dict()
-    assert list(sd_ref.keys()).sort() == list(ours.state_dict().keys()).sort()
-    assert {k: tuple(v.shape) for k, v in sd_ref.items()} == {k: tuple(v.shape) for k, v in ours.state_dict().items()}
-    ours.load_state_dict(sd_ref, strict=True)
-    theirs.load_state_dict(ours.state_dict(), strict=True)
+    assert {k: list(v.shape) for k, v in ours.state_dict().items()} == meta["ncsnpp_v2_shapes"]
+    ours.load_state_dict({k: torch.zeros(s) for k, s in meta["ncsnpp_v2_shapes"].items()}, strict=True)
     # requires_grad flags agree (the Fourier projection is frozen, layerspp.py:37): torch_ema / Adam see the same parameter list
-    assert [(n, p.requires_grad) for n, p in theirs.named_parameters()] == [(n, p.requires_grad) for n, p in ours.named_parameters()]
+    assert [[n, p.requires_grad] for n, p in ours.named_parameters()] == meta["ncsnpp_v2_requires_grad"]
     # same initialisation law: per-tensor standard deviations of a fresh model agree statistically
-    torch.manual_seed(0); a = ref_cls()
-    torch.manual_seed(0); b = cls()
-    for (n, p), (_, q) in zip(a.named_parameters(), b.named_parameters()):
-        if p.numel() > 4096:
-            assert abs(float(p.std()) - float(q.std())) < 0.08 * float(p.std()) + 1e-9, n
+    torch.manual_seed(0)
+    params = dict(cls().named_parameters())
+    stds = meta["ncsnpp_v2_init_std"]
+    assert set(stds) == {n for n, p in params.items() if p.numel() > 4096}
+    for n, s in stds.items():
+        assert abs(float(params[n].detach().std()) - s) < 0.08 * s + 1e-9, n
     # unsupported architecture variants are refused loudly, not silently ignored
     for bad in (dict(dropout=0.1), dict(fir_kernel=[1, 2, 1]), dict(resamp_with_conv=False), dict(progressive="none")):
         with pytest.raises(NotImplementedError):
             cls(**bad)
     pred = R.get_by_name("ncsnpp_v2_predictive_b200")()
-    pred.load_state_dict(R.get_by_name("ncsnpp_v2_predictive")().state_dict(), strict=True)
+    assert {k: list(v.shape) for k, v in pred.state_dict().items()} == meta["ncsnpp_v2_predictive_shapes"]
+    pred.load_state_dict({k: torch.zeros(s) for k, s in meta["ncsnpp_v2_predictive_shapes"].items()}, strict=True)
 
 
-def test_forward_without_cuda_fails_loudly(ref):
+def test_forward_without_cuda_fails_loudly():
     import fdbm_b200
     net = fdbm_b200.NCSNpp_v2()
     x = torch.zeros(1, 1, 257, 64, dtype=torch.complex64)
@@ -75,87 +75,96 @@ def test_forward_without_cuda_fails_loudly(ref):
 
 @pytest.mark.parametrize("path,kw", [("sb", dict(noise_schedule="bb")), ("sb", dict(noise_schedule="ve")),
                                      ("sb", dict(noise_schedule="vp", c=0.3)), ("sb", dict(noise_schedule="gmax")), ("fm", dict())])
-def test_bridge_host_maths_equal_the_reference(ref, path, kw):
+def test_bridge_host_maths_equal_the_reference(golden, path, kw):
     """Attributes callers read / mutate (infer_single.py:55-56, model.py:451-452) and every scalar function of the paths."""
     import fdbm_b200
-    rb = ref["Bridge"](path, N=7, sampler_type="sde_ei", sampling_eps=1e-3, **kw)
+    meta, g = golden
+    tag = f"{path}_{kw.get('noise_schedule', 'ot')}"
+    assert MG.DROPIN_PATHS[tag] == (path, kw)
+    m = meta[tag]
     ob = fdbm_b200.Bridge(path, N=7, sampler_type="sde_ei", sampling_eps=1e-3, **kw)
-    for attr in ("N", "T", "sampler_type", "start_time", "end_time"):
-        assert getattr(rb, attr) == getattr(ob, attr), attr
-    assert rb.path.sampling_direction == ob.path.sampling_direction and rb.path.T == ob.path.T
+    for attr, want in m["attrs"].items():
+        assert as_json(getattr(ob, attr)) == want, attr
+    assert ob.path.sampling_direction == m["sampling_direction"] and ob.path.T == m["path_T"]
     ob.N, ob.sampler_type = 3, "ode_ei"                                           # mutable after construction
     assert ob.time_grid().numel() == 4
-    t = torch.tensor([0.03, 0.2, 0.55, 0.9999, 1.0])
-    for a, b in zip(rb.path.path_param(t), ob.path.path_param(t)):
-        assert torch.equal(a, b)
-    assert torch.equal(rb._std(t), ob._std(t))
-    g = torch.Generator().manual_seed(1)
-    s, y, x = (torch.view_as_complex(torch.randn(5, 1, 9, 4, 2, generator=g)) for _ in range(3))
-    mr, sr = rb.probability_path(s, y, t); mo, so = ob.probability_path(s, y, t)
-    assert torch.equal(mr, mo) and torch.equal(sr, so)
-    assert torch.equal(rb.score_fn(t, x, s, y), ob.score_fn(t, x, s, y))
+
+    def check(name, values, exact=True, rtol=1e-6, atol=1e-7):
+        assert f"{tag}_{name}_{len(values)}" not in g, name
+        for i, v in enumerate(values):
+            got, want = torch.as_tensor(v).numpy(), g[f"{tag}_{name}_{i}"]
+            if exact:
+                assert got.dtype == want.dtype and np.array_equal(got, want), (name, i)
+            else:
+                assert got.shape == want.shape and np.allclose(got, want, rtol=rtol, atol=atol), (name, i)
+
+    t = torch.tensor(MG.DROPIN_T)
+    s, y, x = MG.dropin_bridge_inputs()
+    check("path_param", ob.path.path_param(t))
+    check("std", [ob._std(t)])
+    check("probability_path", ob.probability_path(s, y, t))
+    check("score_fn", [ob.score_fn(t, x, s, y)])
     # ode / sde: the reference's [B]-into-[B,1,F,T] product is only meaningful for B = 1 (its callers); equal there
     t1 = torch.tensor([0.4])
     x1, s1, y1 = x[:1], s[:1], y[:1]
-    assert torch.allclose(rb.path.ode(t1, x1, s1, y1), ob.path.ode(t1, x1, s1, y1), rtol=1e-6, atol=1e-7)
+    check("ode", [ob.path.ode(t1, x1, s1, y1)], exact=False)
     if path == "sb":
-        dr, gr = rb.path.sde(t1, x1, s1, y1); do, go = ob.path.sde(t1, x1, s1, y1)
-        assert torch.allclose(dr, do, rtol=1e-6, atol=1e-7) and torch.allclose(torch.as_tensor(gr), torch.as_tensor(go))
-        fr, g_r = rb.path.auxiliary_param(t1); fo, g_o = ob.path.auxiliary_param(t1)
-        assert torch.allclose(torch.as_tensor(fr, dtype=torch.float32), torch.as_tensor(fo, dtype=torch.float32))
-        assert torch.allclose(torch.as_tensor(g_r), torch.as_tensor(g_o))
-        for st in ("ode_ei", "sde_ei"):
-            fn = "sampling_param_" + st
-            for a, b in zip(getattr(rb.path, fn)(t1 * 0.5, t1, 1, "cpu"), getattr(ob.path, fn)(t1 * 0.5, t1, 1, "cpu")):
-                assert torch.equal(a, b)
+        check("sde", ob.path.sde(t1, x1, s1, y1), exact=False, atol=1e-8)
+        check("auxiliary_param", [torch.as_tensor(v, dtype=torch.float32) for v in ob.path.auxiliary_param(t1)], exact=False,
+              rtol=1e-5, atol=1e-8)
+        check("sampling_param_ode_ei", ob.path.sampling_param_ode_ei(t1 * 0.5, t1, 1, "cpu"))
+        check("sampling_param_sde_ei", ob.path.sampling_param_sde_ei(t1 * 0.5, t1, 1, "cpu"))
     # argparse seam of Bridge and of the path classes
-    for r_cls, o_cls in ((ref["Bridge"], fdbm_b200.Bridge), (type(rb.path), type(ob.path))):
-        pa, pb = argparse.ArgumentParser(), argparse.ArgumentParser()
-        r_cls.add_argparse_args(pa); o_cls.add_argparse_args(pb)
-        assert vars(pa.parse_args([])) == vars(pb.parse_args([]))
+    assert as_json(MG.argparse_defaults(fdbm_b200.Bridge)) == meta["bridge_args"]
+    assert as_json(MG.argparse_defaults(type(ob.path))) == m["path_args"]
 
 
-def test_oracle_pc_and_ode_int_samplers_equal_the_reference(ref):
+def test_oracle_pc_and_ode_int_samplers_equal_the_reference(golden):
     """The oracle's restatement of pc_sampler / ode_sampler_int (the GPU tests' yardstick) against the reference's own
     Bridge, with a cheap stand-in model (B = 1, as the reference's broadcasting requires)."""
     import fdbm_oracle as O
-    g = torch.Generator().manual_seed(3)
-    y = torch.view_as_complex(torch.randn(1, 1, 17, 8, 2, generator=g)) * 0.3
-    model = lambda x, yy, t: 0.6 * x + 0.3 * yy * torch.cos(t)[:, None, None, None] + 0.05 * x.abs()
-    zs = [torch.view_as_complex(torch.randn(1, 1, 17, 8, 2, generator=g)) * 0.5 ** 0.5 for _ in range(40)]
-    for corrector, steps in (("ald", 1), ("langevin", 2), ("none", 1)):
-        for predictor in ("euler_maruyama", "none"):
-            rb = ref["Bridge"]("sb", N=4, sampler_type="pc")
-            ob = O.Bridge("sb", N=4, sampler_type="pc")
-            seq = iter(zs)
-            orig = torch.randn_like
-            torch.randn_like = lambda x, **k: next(seq)
-            try:
-                want = rb.sampler(model, y, predictor_name=predictor, corrector_name=corrector, snr=0.3, corrector_steps=steps)
-            finally:
-                torch.randn_like = orig
-            got = ob.pc_sampler(model, y, predictor_name=predictor, corrector_name=corrector, snr=0.3, corrector_steps=steps,
-                                z0=zs[0], zs=zs[1:])
-            assert torch.allclose(got, want, rtol=1e-5, atol=1e-6), (corrector, predictor)
-    with pytest.raises(ValueError):
-        ref["Bridge"]("sb", N=4, sampler_type="pc").sampler(model, y)             # 'reverse_diffusion' is not registered
-    orig = torch.randn_like
-    torch.randn_like = lambda x, **k: zs[0]
-    try:
-        want = ref["Bridge"]("fm", sampler_type="ode_int").sampler(model, y, rtol=1e-6, atol=1e-6)
-    finally:
-        torch.randn_like = orig
+    _, g = golden
+    y, zs, model = MG.dropin_sampler_inputs()
+    for corrector, steps, predictor in MG.DROPIN_PC:
+        got = O.Bridge("sb", N=4, sampler_type="pc").pc_sampler(model, y, predictor_name=predictor, corrector_name=corrector,
+                                                                 snr=0.3, corrector_steps=steps, z0=zs[0], zs=zs[1:])
+        assert torch.allclose(got, torch.from_numpy(g[f"pc_{corrector}_{predictor}"]), rtol=1e-5, atol=1e-6), (corrector, predictor)
     got = O.Bridge("fm", sampler_type="ode_int").ode_sampler_int(model, y, rtol=1e-6, atol=1e-6, z0=zs[0])
-    assert torch.allclose(got, want, rtol=1e-5, atol=1e-6)
+    assert torch.allclose(got, torch.from_numpy(g["ode_int_fm"]), rtol=1e-5, atol=1e-6)
 
 
-def test_data_module_attributes_and_pad_spec(ref):
+def test_data_module_attributes_and_pad_spec(golden):
     import fdbm_b200
-    rd = ref["SpecsDataModule"](base_dir="/unused", n_fft=512, hop_length=256, num_frames=256, window="sqrthann", gpu=False)
+    meta, g = golden
     od = fdbm_b200.SpecsDataModule(base_dir="/unused", n_fft=512, hop_length=256, num_frames=256, window="sqrthann", gpu=False)
-    for attr in ("normalize", "n_fft", "hop_length", "num_frames", "spec_factor", "spec_abs_exponent", "transform_type"):
-        assert getattr(rd, attr) == getattr(od, attr), attr
-    assert torch.equal(rd.window, od.window)
-    assert set(rd.stft_kwargs) == set(od.stft_kwargs)
+    for attr, want in meta["data_module"].items():
+        assert as_json(getattr(od, attr)) == want, attr
+    assert od.window.numpy().dtype == g["data_module_window"].dtype and np.array_equal(od.window.numpy(), g["data_module_window"])
+    assert sorted(od.stft_kwargs) == meta["data_module_stft_kwargs"]
     with pytest.raises(NotImplementedError):
         fdbm_b200.pad_spec(torch.zeros(1, 1, 257, 10, dtype=torch.complex64), mode="bogus")
+
+
+def test_golden_matches_the_reference(golden):
+    """tests/golden/dropin.npz recomputed from the original project's classes, and our backbones registered into ITS registry with
+    state_dicts interchanged both ways.  Needs a checkout of the original project (FDBM_REFERENCE)."""
+    if not REF or not os.path.isdir(os.path.join(REF, "fdbm")):
+        pytest.skip("needs a checkout of the original project: set FDBM_REFERENCE")
+    import fdbm_b200
+    Bridge, R, SpecsDataModule = MG.import_reference()[:3]
+    meta, g = golden
+    rec = MG.dropin_record(Bridge, R, SpecsDataModule)
+    rmeta = json.loads(str(rec.pop("meta")))
+    ref_std, want_std = rmeta.pop("ncsnpp_v2_init_std"), meta["ncsnpp_v2_init_std"]
+    assert set(ref_std) == set(want_std) and all(abs(ref_std[n] - s) < 0.08 * s + 1e-9 for n, s in want_std.items())
+    assert rmeta == {k: v for k, v in meta.items() if k != "ncsnpp_v2_init_std"}
+    assert set(rec) == set(g)
+    for k, v in rec.items():
+        assert v.shape == g[k].shape and np.allclose(v, g[k], rtol=1e-5, atol=1e-6), k
+    R.register("ncsnpp_v2_b200")(fdbm_b200.NCSNpp_v2)
+    ours, theirs = R.get_by_name("ncsnpp_v2_b200")(), R.get_by_name("ncsnpp_v2")()
+    ours.load_state_dict(theirs.state_dict(), strict=True)
+    theirs.load_state_dict(ours.state_dict(), strict=True)
+    y, _, model = MG.dropin_sampler_inputs()
+    with pytest.raises(ValueError):
+        Bridge("sb", N=4, sampler_type="pc").sampler(model, y)                 # 'reverse_diffusion' is not registered
