@@ -170,11 +170,10 @@ int launch_conv_wgrad(const op_t* dy, int Cout, const op_t* x, int Cin, int ksiz
 int launch_grad_prepare(const float* g, int B, int64_t P, int C, float scale, op_t* g16, float* acc_dst, double* sums, cudaStream_t s,
                         bool acc_first = false, bool sums_prezeroed = false);   // acc_first: acc_dst = value instead of +=
 int launch_gn_bwd_reduce(const op_t* g_a, int g_ld, int g_coff, const void* x, int x16, int C, int C_tot, int c_off,
-                         const float2* tab, const float2* stats, int act, int B, int64_t P, double* S, cudaStream_t s, int b0 = 0);
-// (B, b0): the launch covers utterances b0 .. b0 + B - 1 (all pointers are those of the whole batch)
+                         const float2* tab, const float2* stats, int act, int B, int64_t P, double* S, cudaStream_t s);
 int launch_gn_bwd_apply(const op_t* g_a, int g_ld, int g_coff, const void* x, int x16, int C, int C_tot, int c_off,
                         const float2* tab, const float2* stats, const float* gamma, int act, int B, int64_t P, const double* S,
-                        float* acc_dst, op_t* out16, double* out_sums, cudaStream_t s, bool acc_first = false, int b0 = 0,
+                        float* acc_dst, op_t* out16, double* out_sums, cudaStream_t s, bool acc_first = false,
                         bool sums_prezeroed = false);
 int launch_gn_param_grad(const double* S, int B, int C, float inv_scale, float* dgamma, float* dbeta, cudaStream_t s);
 int launch_gn_stats(const double* sums1, int C1, const double* sums2, int C2, int B, int64_t pixels, float2* stats, cudaStream_t s);

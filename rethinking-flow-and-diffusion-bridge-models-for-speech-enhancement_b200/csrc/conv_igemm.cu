@@ -41,12 +41,8 @@ constexpr int TILE_T = 16, TILE_F = 8;
 constexpr int HALO_T = TILE_T + 2, HALO_F = TILE_F + 2;
 constexpr int A_TILE_BYTES = HALO_T * HALO_F * 128;          // 23040 bytes landed per TMA box
 constexpr int A_TILE_STRIDE = 23552;                         // rounded up to 1024
-#ifndef FDBM_A_STAGES
-#define FDBM_A_STAGES 3
-#define FDBM_B_STAGES 3
-#endif
-constexpr int A_STAGES = FDBM_A_STAGES;
-constexpr int B_STAGES = FDBM_B_STAGES;
+constexpr int A_STAGES = 3;
+constexpr int B_STAGES = 3;
 constexpr int BN = 128;
 constexpr int B_TILE_BYTES = BN * 128;
 constexpr int A_SBO = HALO_F * 128;                          // 1280: distance between 8-pixel row groups
@@ -61,12 +57,6 @@ constexpr int A_TILE1_BYTES = TILE_T * TILE_F * 128;           // 1-tap segments
 // 512 threads start at 128 registers each; setmaxnreg moves registers from the pipeline and transform
 // warpgroups to the two epilogue warpgroups (128 * (56 + 120 + 2 * 168) = 65536)
 constexpr int PIPE_REGS = 56, EPI_REGS = 168, XFORM_REGS = 120;
-#ifndef FDBM_SIDE_RING_DEFAULT
-#define FDBM_SIDE_RING_DEFAULT 1   // fused 1x1 shortcut operands on their own A slot (FDBM_SIDE_RING=0 in the environment: A/B against the single ring)
-#endif
-#ifndef FDBM_EPI_RES2
-#define FDBM_EPI_RES2 1          // 16-bit shortcut rows double-buffered in registers (0: the single-buffer epilogue, 10 % slower on Conv_1)
-#endif
 constexpr int STAGE_BYTES = EPI_GROUPS * 4 * 32 * 32 * 4;       // epilogue transposition tiles, one per warp
 constexpr int STAT_SLOTS = 2;                                  // n-blocks whose statistics a CTA keeps in flight
 constexpr int STAT_BYTES = EPI_GROUPS * 4 * BN * 8;            // per-warp channel (sum, sum of squares) partials
@@ -317,6 +307,9 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
       fence_after_sync();
       uint32_t accumulate = 0;
       const uint32_t d0 = tmem_base + (as * MT) * BN, d1 = d0 + BN;
+      // launches without a side ring keep the plain loop below (and so does the weight producer): walk_steps issues the same
+      // MMAs in the same order, but driving them through it too was measured slower on a B200 at 1000 W (two-segment 3x3
+      // GroupNorm-on-load launches +11-14 %, C -> 4 pyramid launches up to +19 %, 256 x 4 s headline 1320-1326 -> 1278-1292 audio-s/s)
       if (p.side_ring) {
         int step = 0;
         walk_steps(p, [&](bool side, int idx, int tap, int ntaps) {
@@ -380,29 +373,13 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
           const uint32_t b_lo = (sB_lo + (sb * b_stride >> 4)) | lo_const;
           const uint32_t a_lo0 = (a_base0 + a_off) | lo_const, a_lo1 = (a_base1 + a_off) | lo_const;
           if (elect_one()) {
-#ifdef FDBM_MMA_WS
-            // weight-stationary MMAs: the four K-slices of the weight tile are parked in collector buffers b0..b3 by the
-            // MMAs of M-tile 0 and re-used by those of M-tile 1 (one pass over the weight tile in shared memory, not two)
-            if (valid1 && p.bn == BN) {
-              mma_f16_ws<0, 0>(d0, a_hi | (a_lo0 + 0), b_hi | (b_lo + 0), idesc, accumulate);
-              mma_f16_ws<1, 0>(d0, a_hi | (a_lo0 + 2), b_hi | (b_lo + 2), idesc, 1u);
-              mma_f16_ws<2, 0>(d0, a_hi | (a_lo0 + 4), b_hi | (b_lo + 4), idesc, 1u);
-              mma_f16_ws<3, 0>(d0, a_hi | (a_lo0 + 6), b_hi | (b_lo + 6), idesc, 1u);
-              mma_f16_ws<0, 1>(d1, a_hi | (a_lo1 + 0), b_hi | (b_lo + 0), idesc, accumulate);
-              mma_f16_ws<1, 1>(d1, a_hi | (a_lo1 + 2), b_hi | (b_lo + 2), idesc, 1u);
-              mma_f16_ws<2, 1>(d1, a_hi | (a_lo1 + 4), b_hi | (b_lo + 4), idesc, 1u);
-              mma_f16_ws<3, 1>(d1, a_hi | (a_lo1 + 6), b_hi | (b_lo + 6), idesc, 1u);
-            } else
-#endif
-            {
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+              mma_f16(d0, a_hi | (a_lo0 + 2 * k), b_hi | (b_lo + 2 * k), idesc, k == 0 ? accumulate : 1u);
+            if (valid1) {
 #pragma unroll
               for (int k = 0; k < 4; ++k)
-                mma_f16(d0, a_hi | (a_lo0 + 2 * k), b_hi | (b_lo + 2 * k), idesc, k == 0 ? accumulate : 1u);
-              if (valid1) {
-#pragma unroll
-                for (int k = 0; k < 4; ++k)
-                  mma_f16(d1, a_hi | (a_lo1 + 2 * k), b_hi | (b_lo + 2 * k), idesc, k == 0 ? accumulate : 1u);
-              }
+                mma_f16(d1, a_hi | (a_lo1 + 2 * k), b_hi | (b_lo + 2 * k), idesc, k == 0 ? accumulate : 1u);
             }
             mma_commit(b_empty + sb);
             if (tap == ntaps - 1) mma_commit(a_empty + sa);
@@ -429,7 +406,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
     // outside the image stay zero: the convolution pads the *normalised* tensor with zeros.
     // Arithmetic: the affine part in fp32 (an all-16-bit HFMA2 variant was 5% faster but doubled the backbone's
     // error), SiLU(y) = h + h * tanh(h) with h = y/2 (the 1/2 is folded into scale/shift) in packed 16-bit: one
-    // MUFU.TANH per TWO elements.  -DFDBM_XF_EXACT selects fp32 ex2/rcp (A/B reference, ~2x the transform time).
+    // MUFU.TANH per TWO elements (an fp32 ex2/rcp SiLU took ~2x the transform time).
     // The transform shares each SM sub-partition with an epilogue warp and has ~4600 cycles per K-block; the
     // (scale, shift) entries are fetched BEFORE waiting for the tile so that their latency is off the critical path.
     const int tt = threadIdx.x - 256;
@@ -477,13 +454,8 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
               for (int w = 0; w < 4; ++w) {
                 const float2 y = __ffma2_rn(op22f2(h2[w]), sc[j][w], sh[j][w]);
                 if (ACT) {
-#ifdef FDBM_XF_EXACT
-                  const float y0 = 2.0f * y.x, y1 = 2.0f * y.y;
-                  h2[w] = f2op2(__fdividef(y0, 1.0f + __expf(-y0)), __fdividef(y1, 1.0f + __expf(-y1)));
-#else
                   const op2_t h = f2op2(y.x, y.y);
                   h2[w] = __hfma2(h, op2_tanh(h), h);
-#endif
                 } else {
                   h2[w] = f2op2(y.x, y.y);
                 }
@@ -586,23 +558,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
       for (int j = eg; j <= eg; ++j) {
         const TileCoord tc = decode_tile(p, ct * MT + j);
         if (!tc.valid) continue;                          // warp-uniform
-#if defined(FDBM_EPI_TEST)
-        {   // measurement builds only (tools/conv_bench.py): 1 = drain TMEM and discard, 2 = do not even read TMEM
-#if FDBM_EPI_TEST == 1
-          uint32_t acc = 0;
-#pragma unroll
-          for (int ch = 0; ch < BN / 32; ++ch) {
-            uint32_t v[32];
-            tmem_ld_32x32(tmem_base + ((q * 32u) << 16) + (as * MT + j) * BN + ch * 32, v);
-            tmem_ld_wait();
-#pragma unroll
-            for (int u = 0; u < 32; ++u) acc ^= v[u];
-          }
-          if (acc == 0x12345678u && p.out_h16) p.out_h16[0] = op_t(0);
-#endif
-          continue;
-        }
-#endif
         if (do_stats && stat_b != tc.b) {
           if (stat_b >= 0) flush_stats();
           stat_b = tc.b;
@@ -712,12 +667,11 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
         float4 bv = __ldg(reinterpret_cast<const float4*>(bias_p));
         float4 bvb = biasb_p ? __ldg(reinterpret_cast<const float4*>(biasb_p)) : make_float4(0.f, 0.f, 0.f, 0.f);
         float4 res[8];
-#if FDBM_EPI_RES2
         // two register buffers for the 16-bit shortcut rows: chunk ch + 1 is requested BEFORE chunk ch's accumulators are read, a
         // whole chunk ahead of its use (with one buffer the compiler hoisted the fp16 -> fp32 conversions of the freshly requested
-        // rows to the top of the next chunk, in front of the TMEM read and the transposition: the warp sat on the L2 latency there)
+        // rows to the top of the next chunk, in front of the TMEM read and the transposition: the warp sat on the L2 latency there,
+        // and Conv_1 was 10 % slower)
         uint2 res16_buf[2][8];
-#define res16 res16_buf[ch & 1]
         auto load_res16 = [&](int ch) {
           uint2 (&dst)[8] = res16_buf[ch & 1];
           if (full) {
@@ -730,19 +684,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
           }
         };
         if (RES16) load_res16(0);
-#else
-        uint2 res16[8];
-        auto load_res16 = [&](int ch) {
-          if (full) {
-#pragma unroll
-            for (int it = 0; it < 8; ++it) res16[it] = __ldg(reinterpret_cast<const uint2*>(res16_p + roff(it) + ch * 32));
-          } else {
-#pragma unroll
-            for (int it = 0; it < 8; ++it)
-              res16[it] = ((okmask >> it) & 1) ? __ldg(reinterpret_cast<const uint2*>(res16_p + roff(it) + ch * 32)) : make_uint2(0u, 0u);
-          }
-        };
-#endif
         auto load_res = [&](float4 (&r)[8], int ch) {
           if (full) {
 #pragma unroll
@@ -776,14 +717,9 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
           }
           uint32_t v[32];
           tmem_ld_32x32(tmem_base + ((q * 32u) << 16) + (as * MT + j) * BN + ch * 32, v);
-#if FDBM_EPI_RES2
           // (also requesting chunk 0 of the warpgroup's NEXT tile during the last chunk was measured: spills, 5 % slower)
           if (RES16) { if (ch + 1 < n_chunks) load_res16(ch + 1); }
           else if (res_p) load_res(res, ch);
-#else
-          if (RES16) { if (ch == 0) load_res16(0); }      // chunks 1..3 were requested while the previous chunk was stored
-          else if (res_p) load_res(res, ch);
-#endif
           tmem_ld_wait();
 #pragma unroll
           for (int g = 0; g < 8; ++g)
@@ -805,7 +741,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
           for (int it = 0; it < 8; ++it) {
             o_lo[it] = __ffma2_rn(o_lo[it], sc2, bs_lo); o_hi[it] = __ffma2_rn(o_hi[it], sc2, bs_hi);
             if (RES16) {
-              const op2_t* r2 = reinterpret_cast<const op2_t*>(&res16[it]);
+              const op2_t* r2 = reinterpret_cast<const op2_t*>(&res16_buf[ch & 1][it]);
               o_lo[it] = __ffma2_rn(op22f2(r2[0]), sc2, o_lo[it]);
               o_hi[it] = __ffma2_rn(op22f2(r2[1]), sc2, o_hi[it]);
             } else if (res_p) {
@@ -823,11 +759,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
               o_hi[it].y += cbias.w + cw[3].x * p0 + cw[3].y * p1 + cw[3].z * p2 + cw[3].w * p3;
             }
           }
-          // the shortcut registers are free again: request the next chunk's rows now (L2 hits, prefetched one tile ahead), a
-          // whole store + statistics phase ahead of their use, without a second register buffer
-#if !FDBM_EPI_RES2
-          if (RES16 && ch + 1 < n_chunks) load_res16(ch + 1);
-#endif
           float2 ssum_lo = make_float2(0.f, 0.f), ssum_hi = ssum_lo, ssq_lo = ssum_lo, ssq_hi = ssum_lo;
           if (full) {                                       // whole tile inside the image: no per-row predicates
             if (of_p) {
@@ -874,9 +805,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
           __syncwarp();                                   // staging tile is rewritten by the next chunk
           bv = bvn; bvb = bvbn;
         }
-#if FDBM_EPI_RES2
-#undef res16
-#endif
         // (deferring this cross-warp reduction to the start of the warpgroup's next tile -- mbarrier arrive / wait pairs instead
         // of the two bar.sync -- was measured: Conv_1 launches 25 % SLOWER; the barriers keep the four warps of a tile in step)
         if (do_stats) {                                   // block-uniform
@@ -1129,26 +1057,14 @@ int launch_conv_igemm(const ConvArgs& a, cudaStream_t s) {
     // 9-tap blocks first, back to back: the load + transform of each one hides behind the nine taps of the previous
     // one.  (Interleaving the 1-tap blocks between them IN THE SAME RING was measured 5 % slower: the next 9-tap block then
     // has only two short blocks of MMA work to hide behind.  The side ring below interleaves them without that cost.)
-    // FDBM_KSCHED (measurement aid): 1 = 1-tap blocks first, 2 = 1-tap blocks after the first 9-tap block
-    static const int order = getenv("FDBM_KSCHED") ? atoi(getenv("FDBM_KSCHED")) : 0;
     int n = 0;
-    if (order == 1) {
-      for (int i = 0; i < n1; ++i) p.ksched[n++] = one[i];
-      for (int i = 0; i < n9; ++i) p.ksched[n++] = nine[i];
-    } else if (order == 2 && n9 > 0) {
-      p.ksched[n++] = nine[0];
-      for (int i = 0; i < n1; ++i) p.ksched[n++] = one[i];
-      for (int i = 1; i < n9; ++i) p.ksched[n++] = nine[i];
-    } else {
-      for (int i = 0; i < n9; ++i) p.ksched[n++] = nine[i];
-      for (int i = 0; i < n1; ++i) p.ksched[n++] = one[i];
-    }
+    for (int i = 0; i < n9; ++i) p.ksched[n++] = nine[i];
+    for (int i = 0; i < n1; ++i) p.ksched[n++] = one[i];
     for (; n < MAX_KB; ++n) p.ksched[n] = 0;
     // side ring: every 1-tap block is a raw operand without halo (the fused 1x1 shortcut) and there is 9-tap work to hide behind
-    bool side_ok = order == 0 && n1 > 0 && n9 > 0;
+    bool side_ok = n1 > 0 && n9 > 0;
     for (int i = 0; i < a.n_seg; ++i) side_ok = side_ok && (a.seg[i].taps == 9 || !p.seg[i].halo);
-    static const int side_env = getenv("FDBM_SIDE_RING") ? atoi(getenv("FDBM_SIDE_RING")) : FDBM_SIDE_RING_DEFAULT;
-    p.side_ring = side_ok && side_env ? 1 : 0;
+    p.side_ring = side_ok ? 1 : 0;
     p.n_main = p.side_ring ? n9 : kb;
     p.side_gap = p.side_ring ? std::max(3, ceil_div(9 * n9, n1)) : 0;
     p.n_steps = n_kt;

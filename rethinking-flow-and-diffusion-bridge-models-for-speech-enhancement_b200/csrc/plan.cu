@@ -25,8 +25,7 @@ struct Mod {
 
 struct Slot { int64_t off; int64_t numel; bool loaded; };     // fp32 parameter inside `params`
 
-struct Act {                 // one residual-stream tensor [B,T,F,C]: fp32 master, 16-bit GEMM-operand copy, channel sums
-  float* data = nullptr;
+struct Act {                 // one residual-stream tensor [B,T,F,C]: 16-bit GEMM-operand copy, channel sums
   op_t* h16 = nullptr;
   double* sums = nullptr;
   float* grad = nullptr;      // training plans: fp32 gradient accumulator (loss-scaled), zeroed at the start of backward
@@ -312,26 +311,20 @@ struct Builder {
     defer_gn_param(S, Ct, gw_off, gb_off);
     fdbm_plan* plp = P;
     const Act a1 = x1; const Act a2 = x2 ? *x2 : Act();
-    const int cb = gn_chunk(Ct, px);
+    // one reduce + apply launch pair over the whole batch.  Measured: per-utterance chunks small enough for the apply pass to
+    // re-read x and g_a from L2 (level 0) made the level-0 GroupNorm backward 2x SLOWER (1.90 vs 0.93 ms: 64 short launches
+    // with their tails instead of 4).
     bop([=](cudaStream_t s) {
       const bool f1 = plp->grad_first(a1.grad), f2 = C2 ? plp->grad_first(a2.grad) : false;
-      for (int b0 = 0; b0 < B; b0 += cb) {
-        const int nb = std::min(cb, B - b0);
-        if (int rc = launch_gn_bwd_reduce(g_a, Ct, 0, a1.h16, 1, C1, Ct, 0, tab, stats, act, nb, px, S, s, b0)) return rc;
-        if (C2) if (int rc = launch_gn_bwd_reduce(g_a, Ct, C1, a2.h16, 1, C2, Ct, C1, tab, stats, act, nb, px, S, s, b0)) return rc;
-        if (int rc = launch_gn_bwd_apply(g_a, Ct, 0, a1.h16, 1, C1, Ct, 0, tab, stats, gamma, act, nb, px, S, a1.grad, nullptr, nullptr, s, f1, b0)) return rc;
-        if (C2) if (int rc = launch_gn_bwd_apply(g_a, Ct, C1, a2.h16, 1, C2, Ct, C1, tab, stats, gamma, act, nb, px, S, a2.grad, nullptr, nullptr, s, f2, b0)) return rc;
-      }
+      if (int rc = launch_gn_bwd_reduce(g_a, Ct, 0, a1.h16, 1, C1, Ct, 0, tab, stats, act, B, px, S, s)) return rc;
+      if (C2) if (int rc = launch_gn_bwd_reduce(g_a, Ct, C1, a2.h16, 1, C2, Ct, C1, tab, stats, act, B, px, S, s)) return rc;
+      if (int rc = launch_gn_bwd_apply(g_a, Ct, 0, a1.h16, 1, C1, Ct, 0, tab, stats, gamma, act, B, px, S, a1.grad, nullptr, nullptr, s, f1)) return rc;
+      if (C2) if (int rc = launch_gn_bwd_apply(g_a, Ct, C1, a2.h16, 1, C2, Ct, C1, tab, stats, gamma, act, B, px, S, a2.grad, nullptr, nullptr, s, f2)) return rc;
       return FDBM_OK;
     });
   }
-  // utterances per reduce/apply chunk.  Measured: chunks small enough for the apply pass to re-read x and g_a from L2 (one
-  // utterance at level 0) make the level-0 GroupNorm backward 2x SLOWER (1.90 vs 0.93 ms: 64 short launches with their tails
-  // instead of 4), so the whole batch is one chunk; the chunked launch path stays for plans with very large batches.
-  int gn_chunk(int Ct, int64_t px) const { (void)Ct; (void)px; return P->B; }
-  float2* norm_stats(const double* q1, int C1, const double* q2, int C2, int T, int F) {
+  float2* norm_stats(const double* q1) {
     if (!train()) return nullptr;
-    (void)C1; (void)q2; (void)C2; (void)T; (void)F;
     if (q1 != last_stats_q1) return nullptr;            // always called right behind norm_table() of the same GroupNorm (build() checks)
     return last_stats;
   }
@@ -376,7 +369,7 @@ struct Builder {
     if (P->train) a.grad = galloc(static_cast<int64_t>(P->B) * T * F * C);
     return a;
   }
-  void free_act(Act& a) { release(a.data); release(a.h16); if (train()) release(a.sums); a.data = nullptr; a.h16 = nullptr; a.sums = nullptr; }
+  void free_act(Act& a) { release(a.h16); if (train()) release(a.sums); a.h16 = nullptr; a.sums = nullptr; }
   // (scale, shift) table of a GroupNorm over the channel concatenation x1 (+ x2): a tiny launch; the consuming
   // convolution applies it while the operand tile sits in shared memory
   float2* norm_table(const double* q1, int C1, const double* q2, int C2, const float* gamma, const float* beta, int T, int F) {
@@ -493,7 +486,7 @@ struct Builder {
     c0.B = B; c0.T = To; c0.F = Fo; c0.Cout = Cout; c0.out_h16 = h1; c0.sums = h1_sums;
     // the (scale, shift) table of GroupNorm_0 is needed by the on-load path and by every backward pass
     tab0 = norm_table(x1.sums, C1, x2 ? x2->sums : nullptr, C2, g0w, g0b, T, F);
-    float2* stats0 = norm_stats(x1.sums, C1, x2 ? x2->sums : nullptr, C2, T, F);
+    float2* stats0 = norm_stats(x1.sums);
     if (mode == 0) {
       // GroupNorm_0 + SiLU applied by Conv_0 on load, straight from the 16-bit copies of the residual stream
       c0.seg[0] = seg(x1.h16, C1, 9, tab0, Cin, 1); c0.n_seg = 1;
@@ -511,7 +504,7 @@ struct Builder {
     conv_op(c0);
     release(a0); release(tab0);
     float2* tab1 = norm_table(h1_sums, Cout, nullptr, 0, g1w, g1b, To, Fo);
-    float2* stats1 = norm_stats(h1_sums, Cout, nullptr, 0, To, Fo);
+    float2* stats1 = norm_stats(h1_sums);
     Act out = new_act(Cout, To, Fo);
     {
       ConvArgs c;
@@ -527,7 +520,7 @@ struct Builder {
       c.wpack = w1; c.bias = bias1;
       if (!shortcut) c.residual_h16 = x1.h16;
       c.scale = 0.70710678118654752f; c.B = B; c.T = To; c.F = Fo; c.Cout = Cout;
-      c.out_f32 = out.data; c.out_h16 = out.h16; c.sums = out.sums;
+      c.out_h16 = out.h16; c.sums = out.sums;
       if (comb) { c.comb_pyr = comb->pyr; c.comb_w = comb->w; c.comb_b = comb->b; c.comb_C = comb->Cp; }
       conv_op(c);
     }
@@ -592,14 +585,9 @@ struct Builder {
       bop([=](cudaStream_t s) { return launch_groupnorm_act(h1, 1, h1_sums, Cout, nullptr, nullptr, 0, g1w, g1b, B, To, Fo, 1, 0, t2, nullptr, s); });
       { WgradCall w; w.dy = t1; w.dy_ld = Cout; w.Cout = Cout; w.x = t2; w.x_ld = Cout; w.Cin = Cout; w.ksize = 3; w.T = To; w.F = Fo; wgrad_op(w, o_c1w); }
       dgrad_op(t1, Cout, 9, pack_d(o_c1w, Cout, Cout, 3), Cout, To, Fo, t3, nullptr);
-      const int cb1 = gn_chunk(Cout, pxo);
       bop([=](cudaStream_t s) {     // GroupNorm_1 backward: g_h1 (16-bit) + its per-(b,c) sums (Conv_0 bias and FiLM gradients)
-        for (int b0 = 0; b0 < B; b0 += cb1) {            // chunks that fit the L2, see gn_bwd()
-          const int nb = std::min(cb1, B - b0);
-          if (int rc = launch_gn_bwd_reduce(t3, Cout, 0, h1, 1, Cout, Cout, 0, tab1, stats1, 1, nb, pxo, S, s, b0)) return rc;
-          if (int rc = launch_gn_bwd_apply(t3, Cout, 0, h1, 1, Cout, Cout, 0, tab1, stats1, g1w, 1, nb, pxo, S, nullptr, t4, sA1, s, false, b0, true)) return rc;
-        }
-        return FDBM_OK;
+        if (int rc = launch_gn_bwd_reduce(t3, Cout, 0, h1, 1, Cout, Cout, 0, tab1, stats1, 1, B, pxo, S, s)) return rc;
+        return launch_gn_bwd_apply(t3, Cout, 0, h1, 1, Cout, Cout, 0, tab1, stats1, g1w, 1, B, pxo, S, nullptr, t4, sA1, s, false, true);
       });
       // Conv_0: a0 recomputed (or the saved resampled one), wgrad, dgrad, GroupNorm_0 backward into x.grad
       const op_t* a0b = a0;
@@ -637,7 +625,7 @@ struct Builder {
     op_t* w3 = pack(p + "NIN_3.W", C, -1, "", 0, C);
     const int64_t npx = static_cast<int64_t>(B) * T * F;
     float2* tab = norm_table(x.sums, C, nullptr, 0, gw, gb, T, F);
-    float2* stats = norm_stats(x.sums, C, nullptr, 0, T, F);
+    float2* stats = norm_stats(x.sums);
     op_t* qkv = alloc<op_t>(npx * 3 * C);
     {
       ConvArgs c;
@@ -657,7 +645,7 @@ struct Builder {
       c.seg[0] = seg(o, C, 1); c.n_seg = 1;
       c.wpack = w3; c.bias = b3; c.scale = 0.70710678118654752f;
       c.residual_h16 = x.h16;
-      c.B = B; c.T = T; c.F = F; c.Cout = C; c.out_f32 = out.data; c.out_h16 = out.h16; c.sums = out.sums;
+      c.B = B; c.T = T; c.F = F; c.Cout = C; c.out_h16 = out.h16; c.sums = out.sums;
       conv_op(c);
     }
     release(o);
@@ -796,7 +784,7 @@ struct Builder {
       ConvArgs c;
       c.seg[0] = seg(cols, 64, 1); c.n_seg = 1;
       c.wpack = wp; c.bias = b; c.B = B; c.T = T; c.F = F; c.Cout = nf;
-      c.out_f32 = h0.data; c.out_h16 = h0.h16; c.sums = h0.sums;
+      c.out_h16 = h0.h16; c.sums = h0.sums;
       conv_op(c, 2.0 * B * T * F * nf * 9.0 * Cp);
       release(cols);
       if (train()) {
@@ -881,7 +869,7 @@ struct Builder {
         float* pyr_new = alloc<float>(static_cast<int64_t>(B) * Tc * Fc * Cp);
         float* prev = pyramid;
         float2* tab = norm_table(h.sums, C, nullptr, 0, gw, gb, Tc, Fc);
-        float2* stats = norm_stats(h.sums, C, nullptr, 0, Tc, Fc);
+        float2* stats = norm_stats(h.sums);
         ConvArgs c;
         c.seg[0] = seg(h.h16, C, 9, tab, C, 1); c.n_seg = 1;     // GroupNorm + SiLU on load
         c.wpack = wp; c.bias = b; c.B = B; c.T = Tc; c.F = Fc; c.Cout = 16; c.narrow_n = true;

@@ -22,9 +22,7 @@ int launch_clip_rescale(float* wave, int batch, int64_t n_samples, const int* le
                         cudaStream_t s);
 namespace {
 
-// FDBM_SPECTRAL_V1=1 selects the first-generation kernels below (A/B measurements; they are also the path for hops the
-// fast kernels do not cover)
-bool use_v1() { static const bool v = getenv("FDBM_SPECTRAL_V1") && getenv("FDBM_SPECTRAL_V1")[0] == '1'; return v; }
+// The first-generation kernels below serve the hops the fast kernels (spectral_fast.cu) do not cover.
 
 constexpr int NFFT = 512;
 constexpr int NBIN = NFFT / 2 + 1;
@@ -431,7 +429,7 @@ static int stft_launch(const char* who, const float* wave, int batch, int64_t ma
   FDBM_REQUIRE(n_frames_out >= M, "%s: n_frames_out %d < frame count %d", who, n_frames_out, M);
   FDBM_REQUIRE(pad_mode != FDBM_PAD_REFLECTION || n_frames_out - M_min < M_min, "%s: reflection pad wider than the input", who);
   FDBM_REQUIRE(wave && window && spec && wave_stride >= max_samples, "%s: null pointer or bad stride", who);
-  if (spectral_fast_supported(n_fft, hop, false) && !use_v1())
+  if (spectral_fast_supported(n_fft, hop, false))
     return launch_stft_fast(wave, batch, max_samples, lengths, wave_stride, window, norm, hop, transform_type, spec_factor, abs_exponent,
                             pad_mode, M, n_frames_out, spec, as_stream(stream));
   FDBM_REQUIRE(!norm, "%s: the fused peak normalisation needs hop 128 or 256", who);
@@ -471,7 +469,7 @@ static int istft_launch(const char* who, const float* spec, int batch, int n_fra
   FDBM_REQUIRE(batch > 0 && n_frames > 0 && length > 0 && wave_stride >= length, "%s: bad sizes", who);
   FDBM_REQUIRE(transform_type >= 0 && transform_type <= 2, "%s: bad transform", who);
   FDBM_REQUIRE(spec && window && wave, "%s: null pointer", who);
-  if (spectral_fast_supported(n_fft, hop, true) && !use_v1())
+  if (spectral_fast_supported(n_fft, hop, true))
     return launch_istft_fast(spec, batch, n_frames, window, transform_type, spec_factor, abs_exponent, length, lengths, wave_stride, norm,
                              peak, wave, as_stream(stream));
   FDBM_REQUIRE(!norm && !peak, "%s: the fused rescale / peak tracking needs hop = n_fft / 2", who);

@@ -30,22 +30,12 @@ constexpr int NBIN = NFFT / 2 + 1;
 // kernels issue 2.5 x / 4 x fewer instructions than the first generation (ncu: 25.9 M vs 64 M warp instructions for the STFT)
 // but are now latency-bound: ~100 registers per thread allow 16-20 warps per SM, issue slots are 20 % busy, a warp issues
 // every 20 cycles, 37 % of the stall cycles are the block barriers around the staging tile -- larger blocks make that worse,
-// more resident blocks (FDBM_SPEC_MINBLOCKS 5, 6) change nothing or spill.  Dropping the staging tile and its two block barriers
+// more resident blocks (a launch-bounds minimum of 5 or 6 per SM) change nothing or spill.  Dropping the staging tile and its two block barriers
 // (every lane writing the 32 contiguous bytes = 4 frames of its bins straight from registers) was measured too: 1.79 TB/s
 // instead of 2.16 (96 registers), 1.53 with 80 registers / 6 blocks, 1.69 / 1.76 with 8 / 2 warps -- 16-byte pieces of 32
 // different lines per store instruction cost more than the barriers they remove.
-#ifndef FDBM_SPEC_WARPS
-#define FDBM_SPEC_WARPS 4
-#endif
-// FDBM_SPEC_TW_GLOBAL: read the packed twiddle table from global memory (L1-resident, 9 KB) instead of a per-block shared copy;
-// FDBM_SPEC_MINBLOCKS: resident blocks per SM the register allocation must allow
-#ifndef FDBM_SPEC_TW_GLOBAL
-#define FDBM_SPEC_TW_GLOBAL 1
-#endif
-#ifndef FDBM_SPEC_MINBLOCKS
-#define FDBM_SPEC_MINBLOCKS 5
-#endif
-constexpr int FWARPS = FDBM_SPEC_WARPS;
+constexpr int FWARPS = 4;
+constexpr int MIN_BLOCKS = 5;             // resident blocks per SM the register allocation must allow
 constexpr int FPW = 4;                    // frames per warp
 constexpr int FRB = FWARPS * FPW;         // frames per block
 constexpr int LPL = FRB / 2;              // lanes (16-byte pieces = 2 frames) per bin line; 32 * FWARPS / LPL = 16 bins per pass
@@ -59,15 +49,13 @@ __device__ const float2 kTw512[NFFT] = {
 #include "tw512.inc"
 };
 
-__device__ float4 g_tw_packed[2][NFFT + 64];       // [0] forward, [1] inverse (filled once per device)
+// packed-pair twiddles (c, c, s, s) of exp(-+2 pi i m / 512), [0] forward, [1] inverse (filled once per device; read from
+// global memory, L1-resident, 9 KB):  [32 k1 + lane] = W_512^(lane k1) (inter-stage, one row per k1 so that a lane's 15 reads
+// are immediate offsets from one address);  [512 + 16 h + K] = h ? W_32^K : 1 (radix-2 split of the last stage);
+// [544 + M] = W_32^M (the 16-point transform's constants)
+__device__ float4 g_tw_packed[2][NFFT + 64];
 
 struct FastSmem {
-#if !FDBM_SPEC_TW_GLOBAL
-  // packed-pair twiddles (c, c, s, s) of exp(-+2 pi i m / 512):  [32 k1 + lane] = W_512^(lane k1) (inter-stage, one row per k1 so
-  // that a lane's 15 reads are immediate offsets from one address);  [512 + 16 h + K] = h ? W_32^K : 1 (radix-2 split of the last
-  // stage);  [544 + M] = W_32^M (the 16-point transform's constants)
-  float4 tw[NFFT + 64];
-#endif
   union {
     float4 work[FWARPS][WORK_F4];
     float2 tile[NBIN][TILE_PITCH];
@@ -106,7 +94,7 @@ __host__ __device__ constexpr double c32(int m) {
 }
 __host__ __device__ constexpr double s32(int m) { return c32(m - 8); }
 
-// times W_32^M = exp(-+2 pi i M / 32) = tw[16 M]: the packed (c, c, s, s) entry comes from the shared table -- with
+// times W_32^M = exp(-+2 pi i M / 32) = tw[16 M]: the packed (c, c, s, s) entry comes from the twiddle table -- with
 // immediate constants the compiler falls back to scalar FMUL / FFMA (8 instructions per product pair instead of 4 + 1 load)
 template <bool INV, int M>
 DI PC mul_w32(const PC& v, const float4* tw) {
@@ -182,24 +170,12 @@ DI void fft512_pair(PC (&v)[16], float4* work, const float4* tw, int lane) {
 __global__ void fill_tw_global_kernel() {
   for (int m = threadIdx.x; m < NFFT + 64; m += blockDim.x) {
     int idx;
-    if (m < NFFT) idx = ((m & 31) * (m >> 5)) & 511;
-    else if (m < NFFT + 32) idx = m < NFFT + 16 ? 0 : 16 * (m - NFFT - 16);
-    else idx = 16 * (m - NFFT - 32);
-    const float2 w = kTw512[idx];
-    g_tw_packed[0][m] = make_float4(w.x, w.x, w.y, w.y);
-    g_tw_packed[1][m] = make_float4(w.x, w.x, -w.y, -w.y);
-  }
-}
-
-DI void fill_tw(float4* tw, bool inv) {
-  for (int m = threadIdx.x; m < NFFT + 64; m += FWARPS * 32) {
-    int idx;
     if (m < NFFT) idx = ((m & 31) * (m >> 5)) & 511;                       // lane * k1
     else if (m < NFFT + 32) idx = m < NFFT + 16 ? 0 : 16 * (m - NFFT - 16);  // 1 (even lanes) | W_32^K (odd lanes)
     else idx = 16 * (m - NFFT - 32);                                        // W_32^M
     const float2 w = kTw512[idx];
-    const float s = inv ? -w.y : w.y;
-    tw[m] = make_float4(w.x, w.x, s, s);
+    g_tw_packed[0][m] = make_float4(w.x, w.x, w.y, w.y);
+    g_tw_packed[1][m] = make_float4(w.x, w.x, -w.y, -w.y);
   }
 }
 
@@ -234,7 +210,7 @@ DI float compress_scale(float m2, int transform, float factor, float expo, float
 // STFT + compression.  HS = hop / 32 (8 for hop 256, 4 for hop 128).
 // ------------------------------------------------------------------------------------------------------------------
 template <int HS, int MODE>
-__global__ void __launch_bounds__(FWARPS * 32, FDBM_SPEC_MINBLOCKS)
+__global__ void __launch_bounds__(FWARPS * 32, MIN_BLOCKS)
 stft_fast_kernel(const float* __restrict__ wave, int n_samples, const int* __restrict__ lengths, int64_t wave_stride,
                  const float* __restrict__ window, const float* __restrict__ norm, int transform, float factor, float expo,
                  int pad_mode, int M, int n_frames_out, float2* __restrict__ spec) {
@@ -302,13 +278,7 @@ stft_fast_kernel(const float* __restrict__ wave, int n_samples, const int* __res
       __syncwarp();
     }
   }
-#if FDBM_SPEC_TW_GLOBAL
   const float4* twp = g_tw_packed[0];
-#else
-  fill_tw(sm.tw, false);
-  __syncthreads();
-  const float4* twp = sm.tw;
-#endif
   float4* work = sm.u.work[warp];
   if (any) fft512_pair<false>(v, work, twp, lane);
   // Hermitian separation + compression, results kept in registers until every warp has finished reading its exchange buffer
@@ -411,7 +381,7 @@ DI float2 decompress1(float2 z, float inv, int transform, float factor, float ex
 }
 
 template <int MODE>
-__global__ void __launch_bounds__(FWARPS * 32, FDBM_SPEC_MINBLOCKS)
+__global__ void __launch_bounds__(FWARPS * 32, MIN_BLOCKS)
 istft_fast_kernel(const float2* __restrict__ spec, int M, const float* __restrict__ window, int transform, float factor, float expo,
                   int64_t length, const int* __restrict__ lengths, int64_t wave_stride, const float* __restrict__ norm,
                   float* __restrict__ peak, float* __restrict__ wave) {
@@ -447,12 +417,7 @@ istft_fast_kernel(const float2* __restrict__ spec, int M, const float* __restric
       sm.u.tile[k][c] = (m >= 0 && m < M) ? prep(__ldg(in + static_cast<int64_t>(k) * M + m), k) : make_float2(0.f, 0.f);
     }
   }
-#if FDBM_SPEC_TW_GLOBAL
   const float4* twp = g_tw_packed[1];
-#else
-  fill_tw(sm.tw, true);
-  const float4* twp = sm.tw;
-#endif
   __syncthreads();
   // ---- Z_A = F0 + i F1, Z_B = F2 + i F3 with Hermitian extension: bins k > 256 are the conjugates of bin 512 - k
   PC v[16];

@@ -132,28 +132,6 @@ __device__ __forceinline__ void mma_f16(uint32_t tmem_d, uint64_t desc_a, uint64
       ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// Weight-stationary form: the B operand (here: the 128 x 16 weight slice) is kept in collector buffer BUF by a `fill`
-// MMA and re-used by the next MMA on another accumulator (`lastuse`) without a second pass over shared memory.
-// OP: 0 = fill, 1 = lastuse, 2 = discard (no re-use).
-template <int BUF, int OP>
-__device__ __forceinline__ void mma_f16_ws(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                            uint32_t accumulate) {
-#define FDBM_WS_ASM(BUFS, OPS)                                                                               \
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"                                            \
-               "tcgen05.mma.ws.cta_group::1.kind::f16.collector::" BUFS "::" OPS " [%0], %1, %2, %3, p;\n\t}\n" \
-               ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory")
-  if constexpr (OP == 0) {
-    if constexpr (BUF == 0) FDBM_WS_ASM("b0", "fill"); else if constexpr (BUF == 1) FDBM_WS_ASM("b1", "fill");
-    else if constexpr (BUF == 2) FDBM_WS_ASM("b2", "fill"); else FDBM_WS_ASM("b3", "fill");
-  } else if constexpr (OP == 1) {
-    if constexpr (BUF == 0) FDBM_WS_ASM("b0", "lastuse"); else if constexpr (BUF == 1) FDBM_WS_ASM("b1", "lastuse");
-    else if constexpr (BUF == 2) FDBM_WS_ASM("b2", "lastuse"); else FDBM_WS_ASM("b3", "lastuse");
-  } else {
-    if constexpr (BUF == 0) FDBM_WS_ASM("b0", "discard"); else if constexpr (BUF == 1) FDBM_WS_ASM("b1", "discard");
-    else if constexpr (BUF == 2) FDBM_WS_ASM("b2", "discard"); else FDBM_WS_ASM("b3", "discard");
-  }
-#undef FDBM_WS_ASM
-}
 // Arrive on an mbarrier once all previously issued MMAs of this thread have completed.
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))

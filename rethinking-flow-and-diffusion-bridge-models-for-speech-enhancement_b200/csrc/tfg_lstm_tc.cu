@@ -17,7 +17,7 @@
 //     columns are committed in two slices so the first half of the point-wise warps starts while the second slice computes.
 //   * u_s (the unfolded input, 4 taps x 32 channels) is a ring of six single-position tiles [128 seq x 32 ch] (64-byte rows,
 //     SWIZZLE_64B) filled by TMA one position per step; the four taps of a step are four K = 32 UMMA pairs on ring slots.  They
-//     do not depend on h, so step i + 1's are issued right behind step i's commit into the second gate accumulator (EARLY).
+//     do not depend on h, so step i + 1's are issued right behind step i's commit into the second gate accumulator.
 //   * the bias rides in the GEMM: column 120 of the h tile is the constant 1, that row of W_hh holds b_ih + b_hh.  The rows of
 //     the i, f, o gates are pre-scaled by 1/2 (exact): sigmoid(x) = 0.5 tanh(x / 2) + 0.5 costs one MUFU and no multiply.
 //   * ConvTranspose1d: y_{s-1} = h_{s-1} W_lin is issued together with the gates of step s (both read h_{s-1}); a point-wise
@@ -26,7 +26,6 @@
 //   * accumulators: gates 2 x 224 + y 64 TMEM columns.  Warp 0: TMA + MMA issue (one elected lane), warp 1: TMEM owner,
 //     warps 2-9: point-wise update (thread = sequence x half of the CTA's units), cell state in registers.
 #include <cuda.h>
-#include <cstdlib>
 #include "common.cuh"
 #include "tc05.cuh"
 
@@ -142,9 +141,8 @@ struct TcArgs {
   __half* y[2];                        // [direction]: [n_seq][L + 3][32], ConvTranspose1d taps overlap-added
 };
 
-// EARLY: the input half of step i + 1's gates (which does not depend on h_i) is issued right behind step i's commit into the
+// The input half of step i + 1's gates (which does not depend on h_i) is issued right behind step i's commit into the
 // second gate accumulator, so it runs under step i's point-wise update.
-template <bool EARLY>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
 lstm_sweep_tc_kernel(const __grid_constant__ CUtensorMap map_x, const TcArgs a) {
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -198,7 +196,7 @@ lstm_sweep_tc_kernel(const __grid_constant__ CUtensorMap map_x, const TcArgs a) 
   const int seq0 = tile * 128;
   // position of load number q (see the sweep order): forward q, reverse (L + 2) - q
   auto pos_of = [&](int q) { return rev ? (L + 2) - q : q; };
-  auto gate_acc = [&](int i) { return tmem_base + (EARLY ? (i & 1) * NG : 0); };
+  auto gate_acc = [&](int i) { return tmem_base + (i & 1) * NG; };
   const uint32_t tmem_y = tmem_base + 2 * NG;
 
   if (warp == 0) {
@@ -242,21 +240,20 @@ lstm_sweep_tc_kernel(const __grid_constant__ CUtensorMap map_x, const TcArgs a) 
                 idesc_y, kk > 0 ? 1u : 0u);
       }
     };
-    const int ahead = EARLY ? 5 : 4;               // loads in flight / resident beyond step i's first position
+    constexpr int ahead = 5;                       // loads in flight / resident beyond step i's first position
     if (elect_one()) for (int q = 0; q < ahead; ++q) load_u(q);
     __syncwarp();
     for (int q = 0; q < 4; ++q) wait_u(q);
     fence_after_sync();
-    if (EARLY) { if (elect_one()) issue_u_part(0); __syncwarp(); }
+    if (elect_one()) issue_u_part(0);
+    __syncwarp();
     for (int i = 0; i < L; ++i) {
       const int mine = static_cast<int>(rank), theirs = mine ^ 1;
-      if (!EARLY && i > 0) wait_u(i + 3);
       // this CTA's own K-block of h_{i-1} is complete first (no transfer): its MMAs run while the peer's K-block is in flight.
       // (h_local also says this CTA's point-wise warps have read their accumulators of step i - 1.)
       if (i > 0) mbar_wait(h_local, (i - 1) & 1);
       fence_after_sync();
       if (elect_one()) {
-        if (!EARLY) issue_u_part(i);
         issue_h_part(i, mine, 0);
         issue_h_part(i, mine, 1);
       }
@@ -277,7 +274,7 @@ lstm_sweep_tc_kernel(const __grid_constant__ CUtensorMap map_x, const TcArgs a) 
         mma_commit_pair(y_done);                                  // = every reader of h_{i-1} (both slices, y) is done
       }
       __syncwarp();
-      if (EARLY && i + 1 < L) {
+      if (i + 1 < L) {
         wait_u(i + 4);
         fence_after_sync();
         if (elect_one()) issue_u_part(i + 1);
@@ -434,19 +431,14 @@ extern "C" int fdbm_tfg_lstm_sweep(const void* xn, int n_seq, int L, const void*
   if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(lstm input [%d,%d,32]) failed: %d", n_seq, L + 3, (int)r); return FDBM_ECUDA; }
   static PerDeviceOnce attr_once;
   if (attr_once.first(current_device()))
-  {
-    FDBM_CUDA(cudaFuncSetAttribute(lstm_sweep_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM));
-    FDBM_CUDA(cudaFuncSetAttribute(lstm_sweep_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM));
-  }
+    FDBM_CUDA(cudaFuncSetAttribute(lstm_sweep_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM));
   TcArgs a;
   a.n_seq = n_seq; a.L = L;
   for (int d = 0; d < 2; ++d)
     for (int rk = 0; rk < 2; ++rk) a.img[d][rk] = reinterpret_cast<const uint8_t*>(packed) + static_cast<int64_t>(2 * d + rk) * W_IMAGE_BYTES;
   a.y[0] = reinterpret_cast<__half*>(y_fw); a.y[1] = reinterpret_cast<__half*>(y_bw);
   dim3 grid(2 * ceil_div(n_seq, 128), 2);
-  static const bool early = !(getenv("FDBM_TFG_LSTM_EARLY") && atoi(getenv("FDBM_TFG_LSTM_EARLY")) == 0);      // measurement toggle
-  if (early) lstm_sweep_tc_kernel<true><<<grid, TC_THREADS, TC_SMEM, as_stream(stream)>>>(map, a);
-  else lstm_sweep_tc_kernel<false><<<grid, TC_THREADS, TC_SMEM, as_stream(stream)>>>(map, a);
+  lstm_sweep_tc_kernel<<<grid, TC_THREADS, TC_SMEM, as_stream(stream)>>>(map, a);
   FDBM_LAUNCH_CHECK();
   return FDBM_OK;
 }

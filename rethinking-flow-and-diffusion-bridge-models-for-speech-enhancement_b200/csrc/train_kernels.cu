@@ -86,7 +86,6 @@ struct GnBwdArgs {
   // apply outputs
   float* acc_dst;                              // fp32 [B,P,C]: += g_x   (or nullptr)
   int acc_first;                               // ... = g_x: the first contribution of this backward pass to that buffer
-  int b0;                                      // first utterance of this launch (grid.y = utterances of the chunk)
   op_t* out16;                                 // 16-bit [B,P,C] = g_x   (or nullptr)
   double* out_sums;                            // [B,C]: += sum_px g_x   (with out16; or nullptr)
   double inv_count;                            // 1 / (channels per group * P)
@@ -105,19 +104,15 @@ __device__ __forceinline__ void load8(const GnBwdArgs& a, int64_t idx8, float (&
 }
 // d SiLU / dy = sg + y sg (1 - sg), sg = sigmoid(y) = 1/2 + tanh(y/2)/2: one MUFU.TANH instead of EX2 + an IEEE division
 // (these passes were instruction-bound, not HBM-bound: the division alone was a third of their instructions)
-#ifndef FDBM_GNBWD_BLOCKS
-#define FDBM_GNBWD_BLOCKS 4      // resident blocks per SM the register allocation must allow
-#endif
-#ifndef FDBM_GNBWD_UNROLL
-#define FDBM_GNBWD_UNROLL 2      // pixels of a thread's lane in flight per loop trip (measured, norm + elementwise part of a 16-crop backward: 1 -> 24.45 ms, 2 -> 24.00; with 3 or 2 blocks per SM and 80 - 96 registers 25.5 - 26.0)
-#endif
+constexpr int GNBWD_BLOCKS = 4;      // resident blocks per SM the register allocation must allow
+constexpr int GNBWD_UNROLL = 2;      // pixels of a thread's lane in flight per loop trip (measured, norm + elementwise part of a 16-crop backward: 1 -> 24.45 ms, 2 -> 24.00; with 3 or 2 blocks per SM and 80 - 96 registers 25.5 - 26.0)
 template <bool APPLY>
-__global__ void __launch_bounds__(256, FDBM_GNBWD_BLOCKS)
+__global__ void __launch_bounds__(256, GNBWD_BLOCKS)
 gn_bwd_kernel(const GnBwdArgs a, int px_per_block) {
   pdl_wait_then_trigger();
   __shared__ float s_m1[32], s_m2[32];
   __shared__ float s_red[256 * 16];
-  const int b = a.b0 + blockIdx.y;
+  const int b = blockIdx.y;
   const int G = min(a.C_tot / 4, 32), cpg = a.C_tot / G;
   if (APPLY) {
     if (threadIdx.x < G) {
@@ -160,8 +155,7 @@ gn_bwd_kernel(const GnBwdArgs a, int px_per_block) {
   for (int j = 0; j < 4; ++j) { s1[j] = make_float2(0.f, 0.f); s2[j] = make_float2(0.f, 0.f); }
   const int64_t p0 = static_cast<int64_t>(blockIdx.x) * px_per_block, p1 = min(a.P, p0 + px_per_block);
   if (pl < npl) {
-    constexpr int kUnroll = FDBM_GNBWD_UNROLL;
-#pragma unroll kUnroll
+#pragma unroll GNBWD_UNROLL
     for (int64_t p = p0 + pl; p < p1; p += npl) {
       const int64_t row = static_cast<int64_t>(b) * a.P + p;
       float xs[8];
@@ -592,9 +586,8 @@ static int gn_bwd_grid(const GnBwdArgs& a, int B, dim3* grid, int* ppb) {
 
 // one source tensor of a (possibly concatenated) GroupNorm: reduce pass.  S must have been zeroed by the caller.
 int launch_gn_bwd_reduce(const op_t* g_a, int g_ld, int g_coff, const void* x, int x16, int C, int C_tot, int c_off,
-                         const float2* tab, const float2* stats, int act, int B, int64_t P, double* S, cudaStream_t s, int b0) {
+                         const float2* tab, const float2* stats, int act, int B, int64_t P, double* S, cudaStream_t s) {
   GnBwdArgs a{};
-  a.b0 = b0;
   a.g_a = g_a; a.g_ld = g_ld; a.g_coff = g_coff; a.x = x; a.x16 = x16; a.C = C; a.C_tot = C_tot; a.c_off = c_off;
   a.tab = tab; a.stats = stats; a.gamma = nullptr; a.act = act; a.P = P; a.S = S;
   dim3 grid; int ppb;
@@ -606,15 +599,14 @@ int launch_gn_bwd_reduce(const op_t* g_a, int g_ld, int g_coff, const void* x, i
 
 int launch_gn_bwd_apply(const op_t* g_a, int g_ld, int g_coff, const void* x, int x16, int C, int C_tot, int c_off,
                         const float2* tab, const float2* stats, const float* gamma, int act, int B, int64_t P, const double* S,
-                        float* acc_dst, op_t* out16, double* out_sums, cudaStream_t s, bool acc_first, int b0, bool sums_prezeroed) {
+                        float* acc_dst, op_t* out16, double* out_sums, cudaStream_t s, bool acc_first, bool sums_prezeroed) {
   GnBwdArgs a{};
-  a.b0 = b0;
   a.g_a = g_a; a.g_ld = g_ld; a.g_coff = g_coff; a.x = x; a.x16 = x16; a.C = C; a.C_tot = C_tot; a.c_off = c_off;
   a.tab = tab; a.stats = stats; a.gamma = gamma; a.act = act; a.P = P; a.S = const_cast<double*>(S);
   a.acc_dst = acc_dst; a.out16 = out16; a.out_sums = out_sums; a.acc_first = acc_first ? 1 : 0;
   const int G = std::min(C_tot / 4, 32);
   a.inv_count = 1.0 / (static_cast<double>(C_tot / G) * static_cast<double>(P));
-  if (out_sums && !sums_prezeroed) FDBM_CUDA(cudaMemsetAsync(out_sums + static_cast<int64_t>(b0) * C, 0, sizeof(double) * B * C, s));
+  if (out_sums && !sums_prezeroed) FDBM_CUDA(cudaMemsetAsync(out_sums, 0, sizeof(double) * B * C, s));
   dim3 grid; int ppb;
   if (int rc = gn_bwd_grid(a, B, &grid, &ppb)) return rc;
   FDBM_CUDA(launch_maybe_pdl(gn_bwd_kernel<true>, grid, dim3(256), 0, s, pdl_enabled() && B <= pdl_batch_limit(), a, ppb));

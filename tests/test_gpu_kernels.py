@@ -96,12 +96,15 @@ def test_hop128_and_log_transform(lib):
     import fdbm_oracle as O
     from fdbm_b200 import SpecsDataModule
     x = torch.randn(3, 9000, generator=torch.Generator().manual_seed(5))
-    for hop, tt in ((128, "exponent"), (256, "log"), (128, "none")):
+    # hop 512 is outside the fast STFT kernels: it runs the first-generation STFT
+    for hop, tt in ((128, "exponent"), (256, "log"), (128, "none"), (512, "exponent")):
         cfg = O.SpecConfig(n_fft=512, hop_length=hop, window="hann", transform_type=tt)
         dm = SpecsDataModule(n_fft=512, hop_length=hop, window="hann", transform_type=tt)
         ref = O.spec_fwd(O.stft(x, cfg), cfg)
         got = dm.spec_fwd(dm.stft(x.cuda()))
         assert rel_l2(got, ref) < 2e-6, (hop, tt)
+        if hop == 512:
+            continue                          # frames without overlap: the Hann window's zeros make the iSTFT undefined
         wref = O.istft(O.spec_back(ref, cfg), cfg, 9000)
         wgot = dm.to_audio(got, 9000)
         assert rel_l2(wgot, wref) < 5e-6, (hop, tt)
