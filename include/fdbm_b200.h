@@ -363,15 +363,98 @@ int fdbm_conv_igemm(const void* in1, int C1, int ksize, const void* in2, int C2,
                     const void* wpack, const float* bias, const float* bias_b, const float* residual,
                     float scale, int batch, int T, int F, int Cout,
                     float* out_f32, void* out_h16, double* sums, void* stream);
-/* The same convolution with GroupNorm(32 groups, eps 1e-6) (+ SiLU when silu != 0) applied to in1 ON LOAD
- * (layerspp.py:242-246,266-268: h = Conv(act(GroupNorm(h)))): in1 is the RAW h16 tensor, sums1 double [B,C1,2]
- * its per-channel sum / sum of squares over T*F pixels (as produced by `sums` of the producing convolution),
- * gamma/beta fp32 [C1].  The tile is normalised in shared memory between the TMA landing and the MMA, so the
- * stand-alone normalisation pass disappears.  `table` is caller-provided scratch of B*C1*2 floats. */
-int fdbm_conv_igemm_gn(const void* in1, int C1, int ksize, const double* sums1, const float* gamma,
-                       const float* beta, int silu, float* table, const void* wpack, const float* bias,
-                       const float* residual, float scale, int batch, int T, int F, int Cout,
-                       float* out_f32, void* out_h16, double* sums, void* stream);
+/* The full convolution launch the backbone plans make, as a descriptor: up to three K segments, each optionally
+ * normalised on load, and every epilogue the plans use.  fdbm_conv_igemm_ex copies the descriptor field for field into
+ * the plans' own launch arguments and launches the same kernel, so a caller reaches exactly the code paths a plan does.
+ *
+ *   out[b,t,f,n] = scale * ( sum_segments sum_taps W . act(seg.in)[b,t+dt-1,f+df-1,:]
+ *                            + bias[n] + bias_b[b * bias_b_stride + n] + residual[b,t,f,n] )  (+ Combine term)
+ *
+ * One K segment (fdbm_conv_seg):
+ *   in          h16 [B,T,F,C] activation tensor
+ *   C           channels, a multiple of 64 (one K-block = 64 channels)
+ *   taps        9 (3x3, zero padding outside the image) or 1 (1x1)
+ *   norm_tab    NULL = raw operand.  Otherwise fp32 pairs (scale, shift): channel c of utterance b is transformed on load
+ *               to x * scale + shift, then SiLU when act != 0, with entry b * tab_stride + c.  Pixels outside the image
+ *               stay zero: the padding is applied to the transformed tensor.  A 1-tap normalised segment is loaded with its
+ *               halo and read at the centre.  fdbm_gn_table builds such a table; two segments may share one table at
+ *               offsets (tab, tab + 2 * C1 floats) with tab_stride = C1 + C2.
+ *   tab_stride  (scale, shift) pairs per utterance row of norm_tab
+ *   act         0 or 1 (SiLU after the transform; ignored for raw segments)
+ *
+ * fdbm_conv_desc:
+ *   struct_bytes    must be sizeof(fdbm_conv_desc); checked before anything else, so a caller with a stale layout gets
+ *                   FDBM_EINVAL and a message instead of a misread pointer
+ *   seg, n_seg      1..3 segments; unused entries are ignored
+ *   wpack           h16 weights packed by fdbm_pack_conv_weights, K-blocks in segment order: w1 covers the leading
+ *                   segments (their channels concatenated), w2 the concatenation of the trailing raw 1-tap segments
+ *   bias            fp32 [Cout], never NULL
+ *   bias_b          fp32 FiLM rows or NULL; row b starts at b * bias_b_stride (stride 0: every utterance uses row 0)
+ *   residual        fp32 [B,T,F,Cout] or NULL
+ *   residual_h16    h16 [B,T,F,Cout] or NULL; not together with residual, comb_pyr or pyr_out
+ *   scale           applied to everything but the Combine term
+ *   B, T, F, Cout   Cout a multiple of the MMA N: 128, or 64 when Cout == 64, or 16 with narrow_n
+ *   out_f32         fp32 [B,T,F,Cout] or NULL;  out_h16 h16 [B,T,F,Cout] or NULL;  at least one output (or pyr_out)
+ *   sums            double [B,Cout,2] or NULL: per-channel (sum, sum of squares) of the fp32 result; Cout <= 256.
+ *                   Zeroed by the call unless sums_prezeroed != 0, in which case the statistics are added to it
+ *   narrow_n        != 0: MMA N = 16, requires Cout == 16 and pyr_out
+ *   pyr_out         fp32 [B,T,F,pyr_C] or NULL: pyramid output = result[..., :pyr_C] + bias[:pyr_C] + FIR-up x2(pyr_prev)
+ *                   (1 <= pyr_C <= 4, Cout == MMA N, no sums, scale not applied)
+ *   pyr_prev        fp32 [B,T/2,F/2,pyr_C] or NULL; requires even T and F
+ *   comb_pyr        fp32 [B,T,F,comb_C] or NULL: out += comb_b[n] + sum_k comb_w[n * comb_C + k] * comb_pyr[b,t,f,k] after
+ *                   `scale` (Combine, layerspp.py:52-59); needs comb_w [Cout,comb_C], comb_b [Cout], 1 <= comb_C <= 4
+ * At most 16 K-blocks in all.  Violations are refused on the host (FDBM_EINVAL, message in fdbm_last_error()) before any
+ * launch. */
+typedef struct fdbm_conv_seg {
+  const void* in;
+  int C;
+  int taps;
+  const float* norm_tab;
+  int tab_stride;
+  int act;
+} fdbm_conv_seg;
+
+typedef struct fdbm_conv_desc {
+  int struct_bytes;
+  fdbm_conv_seg seg[3];
+  int n_seg;
+  const void* wpack;
+  const float* bias;
+  const float* bias_b;
+  int bias_b_stride;
+  const float* residual;
+  const void* residual_h16;
+  float scale;
+  int B, T, F, Cout;
+  float* out_f32;
+  void* out_h16;
+  double* sums;
+  int sums_prezeroed;
+  int narrow_n;
+  float* pyr_out;
+  const float* pyr_prev;
+  int pyr_C;
+  const float* comb_pyr;
+  const float* comb_w;
+  const float* comb_b;
+  int comb_C;
+} fdbm_conv_desc;
+
+int fdbm_conv_igemm_ex(const fdbm_conv_desc* desc, void* stream);
+
+/* (scale, shift) table of GroupNorm(min(Cr/4, 32) groups, eps 1e-6) over the channel concatenation of two tensors, as
+ * the plans build it for normalise-on-load segments (layerspp.py:242-246): scale = gamma * rstd(group),
+ * shift = beta - mean(group) * scale.
+ *   sums1 double [B,C1,2], sums2 double [B,C2,2] or NULL (C2 = 0): per-channel (sum, sum of squares) over `pixels` pixels
+ *   gamma, beta fp32 [C1+C2]
+ *   blk_real    0, or the real channels of every 128-channel block (fdbm_arch.channel_block_real, e.g. 96): groups and
+ *               counts follow the real channel index, padded channels get (0, 0); C1 and C2 multiples of 128.  Cr is the
+ *               number of real channels
+ *   table       fp32 [B, C1+C2, 2]
+ *   stats       fp32 [B, G, 2] per-group (mean, rstd), G = min(Cr/4, 32), or NULL
+ * C1 + C2 <= 512, and Cr divisible into G groups. */
+int fdbm_gn_table(const double* sums1, int C1, const double* sums2, int C2, const float* gamma, const float* beta,
+                  int blk_real, int batch, int64_t pixels, float* table, float* stats, void* stream);
 /* ---- training step (SURVEY section 8 A10): gradients of the convolutions -------------------------------------
  * dgrad: dX = conv(dY, W') with W'[ci][co][df][dt] = W[co][ci][2-df][2-dt] -- pack W with
  * fdbm_pack_conv_weights_dgrad (w fp32 OIHW [Cout,Cin,k,k]; ksize -1: NIN matrix [Cin][Cout]) and call

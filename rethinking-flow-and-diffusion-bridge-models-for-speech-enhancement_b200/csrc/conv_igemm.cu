@@ -1152,27 +1152,28 @@ extern "C" int fdbm_conv_igemm(const void* in1, int C1, int ksize, const void* i
   return launch_conv_igemm(a, as_stream(stream));
 }
 
-// Same convolution with GroupNorm (+SiLU) applied to in1 on load: in1 is the RAW 16-bit tensor, sums1 its
-// per-channel (sum, sum of squares) over `T*F` pixels, gamma/beta the GroupNorm affine.  `table` is caller-provided
-// scratch of B*C1 float2.  Replaces groupnorm_act + conv_igemm for operands that need no resampling.
-extern "C" int fdbm_conv_igemm_gn(const void* in1, int C1, int ksize, const double* sums1, const float* gamma,
-                                  const float* beta, int silu, float* table, const void* wpack, const float* bias,
-                                  const float* residual, float scale, int batch, int T, int F, int Cout, float* out_f32,
-                                  void* out_h16, double* sums, void* stream) {
+// The plans' launch arguments from the C descriptor, field for field: callers reach exactly the launches a plan makes
+extern "C" int fdbm_conv_igemm_ex(const fdbm_conv_desc* d, void* stream) {
+  // first: a caller whose struct layout differs gets a message here, not a misread pointer on the device
+  FDBM_REQUIRE(d && d->struct_bytes == static_cast<int>(sizeof(fdbm_conv_desc)),
+               "fdbm_conv_igemm_ex: struct_bytes %d != sizeof(fdbm_conv_desc) %d: the caller's descriptor layout is out of date",
+               d ? d->struct_bytes : 0, static_cast<int>(sizeof(fdbm_conv_desc)));
   if (int rc = require_sm100()) return rc;
-  FDBM_REQUIRE(in1 && sums1 && gamma && beta && table && wpack && bias && batch > 0 && T > 0 && F > 0,
-               "fdbm_conv_igemm_gn: bad arguments");
-  FDBM_REQUIRE(ksize == 1 || ksize == 3, "fdbm_conv_igemm_gn: ksize must be 1 or 3");
-  float2* tab = reinterpret_cast<float2*>(table);
-  if (int rc = launch_gn_finalize(sums1, C1, nullptr, 0, gamma, beta, batch, static_cast<int64_t>(T) * F, tab, as_stream(stream)))
-    return rc;
+  FDBM_REQUIRE(d->wpack && d->bias && d->B > 0 && d->T > 0 && d->F > 0, "fdbm_conv_igemm_ex: bad arguments");
   ConvArgs a;
-  a.seg[0].in = reinterpret_cast<const op_t*>(in1); a.seg[0].C = C1; a.seg[0].taps = ksize * ksize;
-  a.seg[0].norm_tab = tab; a.seg[0].tab_stride = C1; a.seg[0].act = silu;
-  a.n_seg = 1;
-  a.wpack = reinterpret_cast<const op_t*>(wpack);
-  a.bias = bias; a.residual = residual; a.scale = scale;
-  a.B = batch; a.T = T; a.F = F; a.Cout = Cout;
-  a.out_f32 = out_f32; a.out_h16 = reinterpret_cast<op_t*>(out_h16); a.sums = sums;
+  for (int i = 0; i < MAX_SEG; ++i) {
+    const fdbm_conv_seg& s = d->seg[i];
+    a.seg[i].in = reinterpret_cast<const op_t*>(s.in); a.seg[i].C = s.C; a.seg[i].taps = s.taps;
+    a.seg[i].norm_tab = reinterpret_cast<const float2*>(s.norm_tab); a.seg[i].tab_stride = s.tab_stride; a.seg[i].act = s.act;
+  }
+  a.n_seg = d->n_seg;
+  a.wpack = reinterpret_cast<const op_t*>(d->wpack);
+  a.bias = d->bias; a.bias_b = d->bias_b; a.bias_b_stride = d->bias_b_stride; a.residual = d->residual;
+  a.residual_h16 = reinterpret_cast<const op_t*>(d->residual_h16);
+  a.scale = d->scale; a.B = d->B; a.T = d->T; a.F = d->F; a.Cout = d->Cout;
+  a.out_f32 = d->out_f32; a.out_h16 = reinterpret_cast<op_t*>(d->out_h16);
+  a.sums = d->sums; a.sums_prezeroed = d->sums_prezeroed != 0;
+  a.pyr_out = d->pyr_out; a.pyr_prev = d->pyr_prev; a.pyr_C = d->pyr_C; a.narrow_n = d->narrow_n != 0;
+  a.comb_pyr = d->comb_pyr; a.comb_w = d->comb_w; a.comb_b = d->comb_b; a.comb_C = d->comb_C;
   return launch_conv_igemm(a, as_stream(stream));
 }

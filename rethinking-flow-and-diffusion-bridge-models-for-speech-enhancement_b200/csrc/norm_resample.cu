@@ -596,6 +596,16 @@ extern "C" int fdbm_groupnorm_act(const float* src1, const double* sums1, int C1
                               as_stream(stream));
 }
 
+// the table exactly as the plans build it for a normalise-on-load convolution (norm_table() in plan.cu)
+extern "C" int fdbm_gn_table(const double* sums1, int C1, const double* sums2, int C2, const float* gamma, const float* beta,
+                             int blk_real, int batch, int64_t pixels, float* table, float* stats, void* stream) {
+  if (int rc = require_sm100()) return rc;
+  FDBM_REQUIRE(sums1 && gamma && beta && table && batch > 0 && pixels > 0, "fdbm_gn_table: bad arguments");
+  FDBM_REQUIRE((C2 == 0) == (sums2 == nullptr), "fdbm_gn_table: sums2/C2 mismatch");
+  return launch_gn_finalize(sums1, C1, sums2, C2, gamma, beta, batch, pixels, reinterpret_cast<float2*>(table), as_stream(stream),
+                            blk_real, reinterpret_cast<float2*>(stats));
+}
+
 extern "C" int fdbm_gn_resample_h16(const void* src1, const double* sums1, int C1, const void* src2, const double* sums2,
                                     int C2, const float* gamma, const float* beta, float* table, int batch, int T, int F,
                                     int mode, void* act_out, void* raw_out, void* stream) {

@@ -26,8 +26,8 @@ EXPORTS = [
     "fdbm_lincomb", "fdbm_rk_error_norm",
     "fdbm_plan_create", "fdbm_plan_destroy", "fdbm_plan_load_weights", "fdbm_plan_device_bytes",
     "fdbm_plan_num_launches", "fdbm_ncsnpp_forward", "fdbm_sampler_run", "fdbm_plan_profile_forward",
-    "fdbm_fir_resample", "fdbm_channel_stats", "fdbm_groupnorm_act", "fdbm_gn_resample_h16", "fdbm_conv_igemm", "fdbm_conv_igemm_gn",
-    "fdbm_pack_conv_weights", "fdbm_attention",
+    "fdbm_fir_resample", "fdbm_channel_stats", "fdbm_groupnorm_act", "fdbm_gn_resample_h16", "fdbm_conv_igemm", "fdbm_conv_igemm_ex",
+    "fdbm_gn_table", "fdbm_pack_conv_weights", "fdbm_attention",
     "fdbm_pack_conv_weights_dgrad", "fdbm_conv_wgrad_workspace_bytes", "fdbm_conv_wgrad",
     "fdbm_groupnorm_act_bwd", "fdbm_fir_resample_h16", "fdbm_attention_bwd", "fdbm_adam_ema_step",
     "fdbm_plan_create_train", "fdbm_ncsnpp_backward", "fdbm_plan_param_info", "fdbm_plan_buffers",
@@ -48,6 +48,28 @@ class TensorRef(C.Structure):
 class Arch(C.Structure):
     _fields_ = [("nf", C.c_int), ("n_levels", C.c_int), ("ch_mult", C.c_int * 8), ("num_res_blocks", C.c_int),
                 ("attn_resolution", C.c_int), ("predictive", C.c_int), ("image_size", C.c_int), ("channel_block_real", C.c_int)]
+
+
+class ConvSeg(C.Structure):
+    # `in` of the C struct is a Python keyword: the field is `in_` here (same offset and type)
+    _fields_ = [("in_", C.c_void_p), ("C", C.c_int), ("taps", C.c_int), ("norm_tab", C.c_void_p), ("tab_stride", C.c_int),
+                ("act", C.c_int)]
+
+
+class ConvDesc(C.Structure):
+    """fdbm_conv_desc: one convolution launch as the plans make it (fields documented in include/fdbm_b200.h)."""
+    _fields_ = [("struct_bytes", C.c_int), ("seg", ConvSeg * 3), ("n_seg", C.c_int), ("wpack", C.c_void_p),
+                ("bias", C.c_void_p), ("bias_b", C.c_void_p), ("bias_b_stride", C.c_int), ("residual", C.c_void_p),
+                ("residual_h16", C.c_void_p), ("scale", C.c_float), ("B", C.c_int), ("T", C.c_int), ("F", C.c_int),
+                ("Cout", C.c_int), ("out_f32", C.c_void_p), ("out_h16", C.c_void_p), ("sums", C.c_void_p),
+                ("sums_prezeroed", C.c_int), ("narrow_n", C.c_int), ("pyr_out", C.c_void_p), ("pyr_prev", C.c_void_p),
+                ("pyr_C", C.c_int), ("comb_pyr", C.c_void_p), ("comb_w", C.c_void_p), ("comb_b", C.c_void_p),
+                ("comb_C", C.c_int)]
+
+    def __init__(self, **kw):
+        kw.setdefault("struct_bytes", C.sizeof(ConvDesc))
+        kw.setdefault("scale", 1.0)
+        super().__init__(**kw)
 
 
 _lib = None
@@ -98,7 +120,8 @@ def load() -> C.CDLL:
         "fdbm_groupnorm_act": (i, [p, p, i, p, p, i, p, p, i, i, i, i, i, p, p, p]),
         "fdbm_gn_resample_h16": (i, [p, p, i, p, p, i, p, p, p, i, i, i, i, p, p, p]),
         "fdbm_conv_igemm": (i, [p, i, i, p, i, p, p, p, p, f, i, i, i, i, p, p, p, p]),
-        "fdbm_conv_igemm_gn": (i, [p, i, i, p, p, p, i, p, p, p, p, f, i, i, i, i, p, p, p, p]),
+        "fdbm_conv_igemm_ex": (i, [C.POINTER(ConvDesc), p]),
+        "fdbm_gn_table": (i, [p, i, p, i, p, p, i, i, i64, p, p, p]),
         "fdbm_pack_conv_weights": (i, [p, i, i, p, i, i, p, C.POINTER(i64), p]),
         "fdbm_pack_conv_weights_dgrad": (i, [p, i, i, i, p, C.POINTER(i64), p]),
         "fdbm_conv_wgrad_workspace_bytes": (i64, [i, i, i, i, i, i]),

@@ -47,6 +47,25 @@ def test_no_silent_fallback_without_gpu():
         SpecsDataModule(n_fft=512, hop_length=256, window="sqrthann").stft(torch.zeros(1, 4000))
 
 
+def test_conv_descriptor_size_is_checked_first():
+    """fdbm_conv_igemm_ex refuses a descriptor whose struct_bytes is not the library's sizeof(fdbm_conv_desc) before it
+    looks at the device, so a stale ctypes layout is an error message here rather than a misread pointer on the GPU."""
+    from fdbm_b200 import _lib
+    lib = _lib.load()
+    d = _lib.ConvDesc()
+    d.struct_bytes = ctypes.sizeof(_lib.ConvDesc) - 8
+    rc = lib.fdbm_conv_igemm_ex(ctypes.byref(d), None)
+    msg = lib.fdbm_last_error().decode()
+    assert rc == -1 and "struct_bytes" in msg and "sizeof(fdbm_conv_desc)" in msg, (rc, msg)
+    assert lib.fdbm_conv_igemm_ex(None, None) == -1 and "struct_bytes" in lib.fdbm_last_error().decode()
+    # the right size gets past that check: without a B200 the device check refuses it; with one, the empty descriptor (no
+    # segments) is refused by the launch's own host-side checks, before any launch
+    d = _lib.ConvDesc()
+    rc = lib.fdbm_conv_igemm_ex(ctypes.byref(d), None)
+    msg = lib.fdbm_last_error().decode()
+    assert rc != 0 and "struct_bytes" not in msg, (rc, msg)
+
+
 def test_product_never_imports_oracle():
     pkg = os.path.join(ROOT, "rethinking-flow-and-diffusion-bridge-models-for-speech-enhancement_b200")
     for dirpath, _, files in os.walk(pkg):

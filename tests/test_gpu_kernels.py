@@ -375,9 +375,10 @@ def test_conv_igemm(lib, B, T, Fq, C1, k, C2, Cout, residual, bias_b):
     (1, 20, 12, 256, 3, 256, 1),       # ragged tiles: halo pixels outside the image must stay exactly zero
     (2, 16, 16, 256, 1, 256, 0),       # attention GroupNorm (no activation) + NIN
 ])
-def test_conv_igemm_groupnorm_on_load(lib, B, T, Fq, C1, k, Cout, silu):
+def test_gn_table_then_conv_igemm_ex_on_load(lib, B, T, Fq, C1, k, Cout, silu):
     """conv(act(GroupNorm(x))) with the normalisation applied to the operand tile in shared memory
-    (layerspp.py:242-246): compared with torch GroupNorm -> SiLU -> conv2d in fp64 on the same 16-bit x."""
+    (layerspp.py:242-246): fdbm_gn_table builds the (scale, shift) table, fdbm_conv_igemm_ex applies it on load.
+    Compared with torch GroupNorm -> SiLU -> conv2d in fp64 on the same 16-bit x."""
     g = torch.Generator().manual_seed(B * 100 + T + C1 + k)
     x = (torch.randn(B, C1, Fq, T, generator=g) * 1.7 + 0.4).to(_h16()).float()
     gamma = 1 + 0.1 * torch.randn(C1, generator=g)
@@ -400,9 +401,13 @@ def test_conv_igemm_groupnorm_on_load(lib, B, T, Fq, C1, k, Cout, silu):
     table = torch.empty(B * C1 * 2, device="cuda")
     out = torch.full((B, T, Fq, Cout), float("nan"), device="cuda")
     sums = torch.empty(B, Cout, 2, dtype=torch.float64, device="cuda")
-    _check(lib, lib.fdbm_conv_igemm_gn(xd.data_ptr(), C1, k, sums1.data_ptr(), gd.data_ptr(), bd.data_ptr(), silu,
-                                       table.data_ptr(), wpack.data_ptr(), biasd.data_ptr(), None, 1.0, B, T, Fq,
-                                       Cout, out.data_ptr(), None, sums.data_ptr(), _stream()))
+    from fdbm_b200 import _lib
+    _check(lib, lib.fdbm_gn_table(sums1.data_ptr(), C1, None, 0, gd.data_ptr(), bd.data_ptr(), 0, B, T * Fq, table.data_ptr(),
+                                  None, _stream()))
+    d = _lib.ConvDesc(n_seg=1, wpack=wpack.data_ptr(), bias=biasd.data_ptr(), scale=1.0, B=B, T=T, F=Fq, Cout=Cout,
+                      out_f32=out.data_ptr(), sums=sums.data_ptr())
+    d.seg[0] = _lib.ConvSeg(in_=xd.data_ptr(), C=C1, taps=k * k, norm_tab=table.data_ptr(), tab_stride=C1, act=silu)
+    _check(lib, lib.fdbm_conv_igemm_ex(C.byref(d), _stream()))
     torch.cuda.synchronize()
     got = ntfc_to_nchw(out).cpu()
     assert torch.isfinite(got).all()

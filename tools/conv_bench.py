@@ -36,12 +36,15 @@ for (T, F, C1, k, C2, Cout, res, f32o, sm) in shapes:
     if gn:
         s1 = torch.stack([x1.double().sum((1, 2)), x1.double().pow(2).sum((1, 2))], -1).contiguous()
         gam = torch.ones(C1, device="cuda"); bet = torch.zeros(C1, device="cuda"); tab = torch.empty(B * C1 * 2, device="cuda")
+        d = _lib.ConvDesc(n_seg=1, wpack=wp.data_ptr(), bias=bias.data_ptr(), residual=resid.data_ptr() if res else None,
+                          scale=0.7071, B=B, T=T, F=F, Cout=Cout, out_f32=out.data_ptr() if f32o else None,
+                          out_h16=o16.data_ptr() if o16 is not None else None, sums=sums.data_ptr() if sm else None)
+        d.seg[0] = _lib.ConvSeg(in_=x1.data_ptr(), C=C1, taps=k * k, norm_tab=tab.data_ptr(), tab_stride=C1, act=1)
     def run():
         if gn:
-            rc = lib.fdbm_conv_igemm_gn(x1.data_ptr(), C1, k, s1.data_ptr(), gam.data_ptr(), bet.data_ptr(), 1, tab.data_ptr(),
-                                        wp.data_ptr(), bias.data_ptr(), resid.data_ptr() if res else None, 0.7071, B, T, F, Cout,
-                                        out.data_ptr() if f32o else None, o16.data_ptr() if o16 is not None else None,
-                                        sums.data_ptr() if sm else None, st())
+            rc = lib.fdbm_gn_table(s1.data_ptr(), C1, None, 0, gam.data_ptr(), bet.data_ptr(), 0, B, T * F, tab.data_ptr(), None, st())
+            assert rc == 0, lib.fdbm_last_error()
+            rc = lib.fdbm_conv_igemm_ex(C.byref(d), st())
             assert rc == 0, lib.fdbm_last_error()
             return
         rc = lib.fdbm_conv_igemm(x1.data_ptr(), C1, k, x2.data_ptr() if C2 else None, C2, wp.data_ptr(), bias.data_ptr(), None,
